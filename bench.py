@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """AGCN fwd+bwd sequences/s on B200 (BASELINE.json metric), one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ntu|utd|mmact_imu|utd_rgb]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ntu|utd|mmact_imu|utd_rgb] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (N > 1: batch-sharded replicas + NCCL gradient all-reduce)
 
 A step = zero_grad + forward + cross-entropy + backward (+ gradient all-reduce when N > 1) of the full 10-unit AGCN
@@ -105,6 +105,23 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BUDGET = 60 << 20     # bytes of array data written by --dump-outputs: with the .npy headers, well inside 64 MB
+
+
+def dump_outputs(outdir, arrays):
+    """Writes every array as outdir/<name>.npy.  Past DUMP_BUDGET each array keeps its share of the budget as a fixed, seeded
+    sample of its flattened elements, so that two runs with the same arguments still write the same elements (none of the
+    workloads above gets there: a training step's outputs are about 14 MB)."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    rng = np.random.default_rng(0)
+    for name, a in arrays.items():
+        if total > DUMP_BUDGET:
+            a = a.reshape(-1)[np.sort(rng.choice(a.size, max(1, a.size * DUMP_BUDGET // total), replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
 def build_model(workload, precision, device, recompute=False):
     from fusion_gcn_b200 import modules as M
     m, t, v, c, ncls, gk = WORKLOADS[workload]
@@ -153,11 +170,18 @@ def run_ours(args):
 
     def step(x, y):
         model.zero_grad(set_to_none=True)
-        loss, _ = loss_and_logits(model, loss_fn, x, y)       # fc + cross-entropy as one kernel (Model.loss)
+        loss, logits = loss_and_logits(model, loss_fn, x, y)       # fc + cross-entropy as one kernel (Model.loss)
         loss.backward()
         if reducer is not None:
             reducer()
-        return loss
+        return loss.detach(), logits.detach()       # detached: a kept result must not keep the step's autograd graph alive
+                                                    # (its AccumulateGrad nodes would invalidate the CUDA-graph capture below)
+
+    def step_outputs(loss, logits):
+        """What a caller of the training step receives: the loss, the logits and every parameter gradient."""
+        out = {"loss": loss, "logits": logits}
+        out.update({"grad." + k: p.grad for k, p in model.named_parameters() if p.grad is not None})
+        return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
 
     def barrier():
         if world > 1:
@@ -176,13 +200,15 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(x_dev, y_dev)
+        loss, logits = step(x_dev, y_dev)
     e1.record()
     barrier()
     launches = capi.lib().agcn_launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
     timings = ops.stop_timing()
     ms = e0.elapsed_time(e1)
+    eager_outputs = step_outputs(loss, logits) if args.dump_outputs else None
+    graph_outputs = None
     # ---- end-to-end: host pinned buffers -> device every step, loss read back every step
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -190,7 +216,7 @@ def run_ours(args):
     for _ in range(args.steps):
         xb = x_host.to(dev, non_blocking=True)
         yb = y_host.to(dev, non_blocking=True)
-        loss_val = step(xb, yb).item()
+        loss_val = step(xb, yb)[0].item()
     f1.record()
     barrier()
     ms_e2e = f0.elapsed_time(f1)
@@ -212,6 +238,7 @@ def run_ours(args):
             h1.record()
             barrier()
             ms_graph = h0.elapsed_time(h1)
+            graph_outputs = step_outputs(gs.loss, gs.logits) if args.dump_outputs else None
             e2e_path = None
             nbar = 0                                     # barriers passed inside the try: a rank that falls back must not add any
             try:
@@ -326,6 +353,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, graph_outputs if graph_ok else eager_outputs)
     pk = peaks()
     n_global = n_local * world
     # headline: the step replayed as one CUDA graph (the package's GraphedStep) when every rank captured it, else the eager launches
@@ -496,13 +525,15 @@ def run_infer(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(x_dev)
+        logits = step(x_dev)
     e1.record()
     barrier()
     launches = capi.lib().agcn_launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
     timings = ops.stop_timing()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": logits.float().cpu().numpy()})
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     f0.record()
@@ -621,7 +652,7 @@ def run_reference(args):
     if rank != 0:
         return
     m, t, v, c, ncls, _ = WORKLOADS[args.workload]
-    steps = max(5, min(args.steps, 8))
+    steps = args.steps
     base = cpu_reference(args.workload, steps=steps, warmup=max(1, min(args.warmup, 2)))
     line = {"impl": "reference", "metric": "AGCN fwd+bwd sequences/sec", "value": base["value"], "unit": "sequences/s",
             "n_gpus": args.gpus, "steps": steps, "warmup": max(1, min(args.warmup, 2)), "ms_per_step": base["ms_per_step"],
@@ -655,7 +686,12 @@ def main():
     ap.add_argument("--recompute", action="store_true", help="activation-recompute policy (modules.set_recompute): less memory, two more launches per unit")
     ap.add_argument("--no-graph", action="store_true", help="skip the CUDA-graph replay timing")
     ap.add_argument("--no-tf32", action="store_true", help="skip the extra TF32-mode timing that the fp32 run reports beside the headline")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the headline path computed in its last step as DIR/<name>.npy (float32): "
+                         "loss, logits and every parameter gradient (grad.<parameter>); --mode infer: the logits")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this package's timed path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.batch is None:

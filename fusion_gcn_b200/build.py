@@ -1,5 +1,6 @@
 """Builds libagcn_b200.so in-tree with nvcc for sm_100a:  python -m fusion_gcn_b200.build [--force]"""
 import os
+import shutil
 import subprocess
 import sys
 
@@ -19,11 +20,25 @@ def _stale():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
+def _nvcc():
+    """$NVCC, else nvcc on PATH, else the toolkit's own (CUDA_HOME, CUDA_PATH, the default install prefix): a login shell
+    need not have the toolkit's bin directory on PATH."""
+    if os.environ.get("NVCC"):
+        return os.environ["NVCC"]
+    found = shutil.which("nvcc")
+    if found:
+        return found
+    for root in (os.environ.get("CUDA_HOME"), os.environ.get("CUDA_PATH"), "/usr/local/cuda"):
+        if root and os.path.isfile(os.path.join(root, "bin", "nvcc")):
+            return os.path.join(root, "bin", "nvcc")
+    raise RuntimeError("nvcc not found: put it on PATH, or set NVCC or CUDA_HOME")
+
+
 def build(force=False, verbose=False, probes=False):
     """``probes=True`` compiles the A/B switches and limiter probes in (-DAGCN_PROBES); the default library has none."""
     if not force and not probes and not _stale():
         return OUT
-    nvcc = os.environ.get("NVCC", "nvcc")
+    nvcc = _nvcc()
     out = OUT.replace(".so", "_probes.so") if probes else OUT        # the probe build never replaces the product library
     cmd = [nvcc] + FLAGS + (["-DAGCN_PROBES"] if probes else []) + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES] + ["-lcuda"]
     res = subprocess.run(cmd, capture_output=True, text=True)
