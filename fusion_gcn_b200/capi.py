@@ -46,23 +46,17 @@ SIGNATURES = {
     "agcn_bn_stats": (_c_int, [_c_void_p, _c_int, _c_int, _c_ll, _c_int] + [_c_void_p] * 5 + [_c_float, _c_float, _c_int]
                       + [_c_void_p] * 4 + [_c_void_p, _c_size_t, _c_void_p]),
     "agcn_bn_finalize": (_c_int, [_c_void_p, _c_int, _c_ll, _c_int] + [_c_void_p] * 5 + [_c_float, _c_float] + [_c_void_p] * 5),
-    "agcn_bn_apply": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int, _c_void_p, _c_int, _c_int, _c_ll, _c_int, _c_void_p]),
+    "agcn_bn_apply": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int, _c_int, _c_ll, _c_int, _c_void_p]),
     "agcn_bn_mask_words": (_c_size_t, [_c_int] * 3),
-    "agcn_bn_apply_mask": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int, _c_void_p, _c_void_p, _c_int, _c_int, _c_void_p]),
-    "agcn_bn_apply_mask_split": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int, _c_int, _c_void_p]),
-    "agcn_bn_bwd_bits_split": (_c_int, [_c_void_p] * 11 + [_c_int, _c_int, _c_int, _c_int, _c_void_p, _c_size_t, _c_void_p]),
-    "agcn_bn_bwd_bits": (_c_int, [_c_void_p] * 10 + [_c_int, _c_int, _c_int, _c_int, _c_void_p, _c_size_t, _c_void_p]),
-    "agcn_bn_bwd": (_c_int, [_c_void_p] * 10 + [_c_int, _c_int, _c_int, _c_int, _c_ll, _c_int, _c_void_p, _c_size_t, _c_void_p]),
+    "agcn_bn_bwd": (_c_int, [_c_void_p] * 12 + [_c_int, _c_int, _c_int, _c_int, _c_ll, _c_int, _c_int, _c_int, _c_void_p, _c_double,
+                             _c_void_p, _c_size_t, _c_void_p]),
     "agcn_pool_fwd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p]),
     "agcn_pool_bwd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p]),
     "agcn_bn_apply_pool_workspace_bytes": (_c_size_t, [_c_int, _c_int]),
     "agcn_bn_apply_pool": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p, _c_size_t, _c_void_p]),
-    "agcn_bn_bwd_pool": (_c_int, [_c_void_p] * 11 + [_c_int, _c_int, _c_int, _c_int, _c_void_p, _c_size_t, _c_void_p]),
     "agcn_bn_bwd_bits_dual": (_c_int, [_c_void_p] * 17 + [_c_int, _c_int, _c_int, _c_void_p, _c_size_t, _c_void_p]),
     "agcn_bn_stats_partials_bytes": (_c_size_t, [_c_int]),
     "agcn_bn_stats_partials": (_c_int, [_c_void_p, _c_int, _c_int, _c_ll, _c_int, _c_void_p, _c_size_t, _c_void_p, _c_void_p, _c_size_t, _c_void_p]),
-    "agcn_bn_bwd_sync": (_c_int, [_c_void_p] * 12 + [_c_int, _c_int, _c_int, _c_ll, _c_int, _c_int, _c_int, _c_void_p, _c_double,
-                                  _c_void_p, _c_size_t, _c_void_p]),
     "agcn_linear_ce_fwd": (_c_int, [_c_void_p] * 8 + [_c_int] * 3 + [_c_void_p]),
     "agcn_linear_ce_bwd": (_c_int, [_c_void_p] * 7 + [_c_int] * 3 + [_c_void_p]),
     "agcn_node_mix": (_c_int, [_c_void_p, _c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_int, _c_int, _c_void_p]),

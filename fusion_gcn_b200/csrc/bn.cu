@@ -76,7 +76,7 @@ __device__ __forceinline__ unsigned mask_nibble(const unsigned* bits, long long 
 }
 
 // bcast_rows > 0 (MODE 1): dout is the gradient of a fused mean pool, [groups][channels]; element (r, c) reads
-// dout[r / bcast_rows][c] * bcast_scale (agcn_bn_bwd_pool).
+// dout[r / bcast_rows][c] * bcast_scale (agcn_bn_bwd with pool_rows > 0).
 template <int MODE>
 __global__ void __launch_bounds__(256) colsum_vec_kernel(const float* x, const float* dout, const float* mask, const unsigned* mask_bits,
                                                          const float* mean, const float* invstd,
@@ -716,18 +716,21 @@ extern "C" AGCN_API int agcn_bn_finalize(const float* part, int nparts, long lon
 }
 
 extern "C" AGCN_API size_t agcn_bn_mask_words(int outer, int inner, int channels) {
-    // one bit per element of a CONTIGUOUS [rows][channels] tensor; only layouts both the writer (agcn_bn_apply_mask) and the
-    // reader (agcn_bn_bwd_bits) vectorise are supported -- 0 otherwise (use the fp32 tensor as the mask then)
+    // one bit per element of a CONTIGUOUS [rows][channels] tensor; only layouts both the writer (agcn_bn_apply) and the
+    // reader (agcn_bn_bwd) vectorise are supported -- 0 otherwise (use the fp32 tensor as the mask then)
     if (outer != 1 || inner <= 0 || channels <= 0) return 0;
     RowMap m{1, inner, 0, channels};
     if (!colsum_vec_shape(m)) return 0;
     return (size_t)(((long long)inner * channels + 31) / 32);
 }
 
-static int bn_apply_impl(const float* y, const float* scale, const float* shift,
-                         int res_mode, const float* res, const float* scale2, const float* shift2,
-                         int relu, float* out, unsigned* mask_bits, int outer, int inner, long long outer_stride, int channels, void* stream,
-                         unsigned short* split = nullptr) {
+// mask_bits / out_split (NULL: not written): the ReLU mask as one bit per element and `out` as bf16 pieces [2][inner][channels]
+// (plane 0 = h = bf16(out), plane 1 = m = bf16(out - h)), the operand format of agcn_conv_wgrad_presplit -- the weight gradient of
+// the convolution that consumes `out` then needs no conversion pass of its own.
+extern "C" AGCN_API int agcn_bn_apply(const float* y, const float* scale, const float* shift,
+                                      int res_mode, const float* res, const float* scale2, const float* shift2,
+                                      int relu, float* out, unsigned* mask_bits, void* out_split,
+                                      int outer, int inner, long long outer_stride, int channels, void* stream) {
     int rc = check_map("agcn_bn_apply", outer, inner, outer_stride, channels);
     if (rc) return rc;
     AGCN_REQUIRE(y && scale && shift && out, AGCN_ERR_NULL, "agcn_bn_apply: null pointer");
@@ -737,12 +740,13 @@ static int bn_apply_impl(const float* y, const float* scale, const float* shift,
     RowMap m{outer, inner, outer_stride, channels};
     const long long rows = (long long)outer * inner;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
+    unsigned short* split = static_cast<unsigned short*>(out_split);
     const bool vec = vec_ok(m, {y, scale, shift, res, scale2, shift2, out});
     if (mask_bits != nullptr)
         AGCN_REQUIRE(vec && agcn_bn_mask_words(outer, inner, channels) > 0, AGCN_ERR_UNSUPPORTED,
-                     "agcn_bn_apply_mask: layout not supported (agcn_bn_mask_words returned 0)");
+                     "agcn_bn_apply: mask_bits: layout not supported (agcn_bn_mask_words returned 0)");
     if (split != nullptr)
-        AGCN_REQUIRE(vec && outer == 1 && aligned16(split), AGCN_ERR_UNSUPPORTED, "agcn_bn_apply_mask_split: contiguous, vectorisable layout required");
+        AGCN_REQUIRE(vec && outer == 1 && aligned16(split), AGCN_ERR_UNSUPPORTED, "agcn_bn_apply: out_split needs a contiguous, vectorisable layout");
     if (vec)
         bn_apply_kernel<true><<<elementwise_blocks(rows * (channels / 4)), 256, 0, s>>>(y, scale, shift, res_mode, res, scale2, shift2, relu, out, mask_bits, m, rows, split);
     else
@@ -750,41 +754,26 @@ static int bn_apply_impl(const float* y, const float* scale, const float* shift,
     return check_launch("agcn_bn_apply");
 }
 
-extern "C" AGCN_API int agcn_bn_apply(const float* y, const float* scale, const float* shift,
-                             int res_mode, const float* res, const float* scale2, const float* shift2,
-                             int relu, float* out, int outer, int inner, long long outer_stride, int channels, void* stream) {
-    return bn_apply_impl(y, scale, shift, res_mode, res, scale2, shift2, relu, out, nullptr, outer, inner, outer_stride, channels, stream);
-}
-
-extern "C" AGCN_API int agcn_bn_apply_mask(const float* y, const float* scale, const float* shift,
-                                  int res_mode, const float* res, const float* scale2, const float* shift2,
-                                  int relu, float* out, unsigned* mask_bits, int inner, int channels, void* stream) {
-    AGCN_REQUIRE(mask_bits, AGCN_ERR_NULL, "agcn_bn_apply_mask: null mask pointer");
-    return bn_apply_impl(y, scale, shift, res_mode, res, scale2, shift2, relu, out, mask_bits, 1, inner, 0, channels, stream);
-}
-
-// agcn_bn_apply_mask that also writes `out` as bf16 pieces: out_split [2][inner][channels] (plane 0 = h = bf16(out), plane 1 =
-// m = bf16(out - h)), the operand format of agcn_conv_wgrad_presplit -- the weight gradient of the convolution that consumes `out`
-// then needs no conversion pass of its own.
-extern "C" AGCN_API int agcn_bn_apply_mask_split(const float* y, const float* scale, const float* shift,
-                                                 int res_mode, const float* res, const float* scale2, const float* shift2,
-                                                 int relu, float* out, unsigned* mask_bits, void* out_split, int inner, int channels, void* stream) {
-    AGCN_REQUIRE(mask_bits && out_split, AGCN_ERR_NULL, "agcn_bn_apply_mask_split: null pointer");
-    return bn_apply_impl(y, scale, shift, res_mode, res, scale2, shift2, relu, out, mask_bits, 1, inner, 0, channels, stream,
-                         static_cast<unsigned short*>(out_split));
-}
-
-static int bn_bwd_impl(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
-                       const float* save_mean, const float* save_invstd, const float* gamma,
-                       float* dy, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
-                       int outer, int inner, long long outer_stride, int channels,
-                       void* workspace, size_t workspace_bytes, void* stream, int bcast_rows = 0, int frozen = 0, unsigned short* dy_split = nullptr,
-                       int phase = 0, const float* global_sums = nullptr, double global_rows = 0.0) {
-    // phase 0: the whole backward.  Synchronised BatchNorm (statistics over all ranks) splits it around the caller's all-reduce:
-    // phase 1 = column sums only (dbeta = sum g, dgamma = sum g xhat of THIS rank's rows), phase 2 = the apply pass from
-    // global_sums [2][C] = (sum g | sum g xhat) over all ranks and the global row count.
+// phase 0: the whole backward.  Synchronised BatchNorm (statistics over all ranks) splits it around the caller's all-reduce:
+// phase 1 = column sums only (dbeta = sum g, dgamma = sum g xhat of THIS rank's rows), phase 2 = the apply pass from
+// global_sums [2][C] = (sum g | sum g xhat) over all ranks and the global row count.
+// pool_rows > 0: dout is the gradient of the fused mean pool, [inner / pool_rows][C], broadcast over the rows of each group.
+extern "C" AGCN_API int agcn_bn_bwd(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
+                                    const float* save_mean, const float* save_invstd, const float* gamma,
+                                    float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
+                                    int frozen_stats, int outer, int inner, long long outer_stride, int channels, int pool_rows,
+                                    int phase, const float* global_sums, double global_rows,
+                                    void* workspace, size_t workspace_bytes, void* stream) {
     int rc = check_map("agcn_bn_bwd", outer, inner, outer_stride, channels);
     if (rc) return rc;
+    AGCN_REQUIRE(phase >= 0 && phase <= 2, AGCN_ERR_UNSUPPORTED, "agcn_bn_bwd: phase %d", phase);
+    AGCN_REQUIRE(!frozen_stats || (pool_rows == 0 && phase == 0), AGCN_ERR_UNSUPPORTED,
+                 "agcn_bn_bwd: frozen statistics take neither a pooled gradient nor the synchronised phases");
+    AGCN_REQUIRE(!(mask_out && mask_bits), AGCN_ERR_UNSUPPORTED, "agcn_bn_bwd: mask_out and mask_bits are alternatives, not both");
+    AGCN_REQUIRE(phase != 1 || (dgamma && dbeta), AGCN_ERR_NULL, "agcn_bn_bwd: phase 1 writes dgamma / dbeta");
+    AGCN_REQUIRE(!dy_split || dy, AGCN_ERR_NULL, "agcn_bn_bwd: dy_split needs dy");
+    AGCN_REQUIRE(pool_rows >= 0 && (pool_rows == 0 || (outer == 1 && inner % pool_rows == 0)), AGCN_ERR_BAD_SHAPE, "agcn_bn_bwd: bad pooled shape");
+    AGCN_REQUIRE(pool_rows == 0 || mask_bits, AGCN_ERR_NULL, "agcn_bn_bwd: a pooled gradient needs mask_bits");
     AGCN_REQUIRE(dout && y && save_mean && save_invstd && workspace, AGCN_ERR_NULL, "agcn_bn_bwd: null pointer");
     AGCN_REQUIRE(workspace_bytes >= agcn_bn_workspace_bytes(channels), AGCN_ERR_WORKSPACE, "agcn_bn_bwd: workspace too small");
     RowMap m{outer, inner, outer_stride, channels};
@@ -792,60 +781,33 @@ static int bn_bwd_impl(const float* dout, const float* mask_out, const unsigned*
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     float* part = static_cast<float*>(workspace);
     float* coef = part + (size_t)kMaxPartials * 2 * channels;
+    unsigned short* split = static_cast<unsigned short*>(dy_split);
     const int P = num_partials(rows);
     if (mask_bits != nullptr)
         AGCN_REQUIRE(agcn_bn_mask_words(outer, inner, channels) > 0 && vec_ok(m, {dout, y, dy, dres, workspace}), AGCN_ERR_UNSUPPORTED,
-                     "agcn_bn_bwd_bits: layout not supported (agcn_bn_mask_words returned 0)");
-    const float bcast_scale = bcast_rows > 0 ? 1.f / (float)bcast_rows : 1.f;
+                     "agcn_bn_bwd: mask_bits: layout not supported (agcn_bn_mask_words returned 0)");
+    const float bcast_scale = pool_rows > 0 ? 1.f / (float)pool_rows : 1.f;
     if (phase == 2) {
-        AGCN_REQUIRE(global_sums && global_rows >= (double)rows, AGCN_ERR_NULL, "agcn_bn_bwd_sync: phase 2 needs the all-reduced sums and the global row count");
+        AGCN_REQUIRE(global_sums && global_rows >= (double)rows, AGCN_ERR_NULL, "agcn_bn_bwd: phase 2 needs the all-reduced sums and the global row count");
         bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(global_sums, 1, channels, global_rows, gamma, save_mean, save_invstd,
-                                                                                         nullptr, nullptr, coef, frozen);
+                                                                                         nullptr, nullptr, coef, frozen_stats);
     } else {
-        rc = launch_colsum<1>(y, dout, mask_out, save_mean, save_invstd, m, rows, part, P, s, mask_bits, bcast_rows, bcast_scale);
+        rc = launch_colsum<1>(y, dout, mask_out, save_mean, save_invstd, m, rows, part, P, s, mask_bits, pool_rows, bcast_scale);
         if (rc) return rc;
-        bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part, P, channels, (double)rows, gamma, save_mean, save_invstd, dgamma, dbeta, coef, frozen);
+        bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part, P, channels, (double)rows, gamma, save_mean, save_invstd, dgamma, dbeta, coef, frozen_stats);
     }
     rc = check_launch("agcn_bn_bwd(finalize)");
     if (rc) return rc;
     if (phase == 1 || (dy == nullptr && dres == nullptr)) return AGCN_OK;
-    if (dy_split != nullptr)
-        AGCN_REQUIRE(dy != nullptr && outer == 1 && aligned16(dy_split) && vec_ok(m, {dout, mask_out, y, dy, dres, coef}), AGCN_ERR_UNSUPPORTED,
-                     "agcn_bn_bwd_bits_split: contiguous, vectorisable layout and a dy output required");
+    if (split != nullptr)
+        AGCN_REQUIRE(outer == 1 && aligned16(split) && vec_ok(m, {dout, mask_out, y, dy, dres, coef}), AGCN_ERR_UNSUPPORTED,
+                     "agcn_bn_bwd: dy_split needs a contiguous, vectorisable layout");
     if (vec_ok(m, {dout, mask_out, y, dy, dres, coef}))
         bn_bwd_apply_kernel<true><<<elementwise_blocks(rows * (channels / 4)), 256, 0, s>>>(dout, mask_out, mask_bits, y, coef, dy, dres, dres_accumulate, m, rows,
-                                                                                            bcast_rows, bcast_scale, dy_split);
+                                                                                            pool_rows, bcast_scale, split);
     else
         bn_bwd_apply_kernel<false><<<elementwise_blocks(rows * channels), 256, 0, s>>>(dout, mask_out, nullptr, y, coef, dy, dres, dres_accumulate, m, rows);
     return check_launch("agcn_bn_bwd(apply)");
-}
-
-extern "C" AGCN_API int agcn_bn_bwd(const float* dout, const float* mask_out, const float* y,
-                           const float* save_mean, const float* save_invstd, const float* gamma,
-                           float* dy, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                           int outer, int inner, long long outer_stride, int channels,
-                           void* workspace, size_t workspace_bytes, void* stream) {
-    return bn_bwd_impl(dout, mask_out, nullptr, y, save_mean, save_invstd, gamma, dy, dgamma, dbeta, dres, dres_accumulate,
-                       outer, inner, outer_stride, channels, workspace, workspace_bytes, stream, 0, frozen_stats);
-}
-
-extern "C" AGCN_API int agcn_bn_bwd_bits(const float* dout, const unsigned* mask_bits, const float* y,
-                                const float* save_mean, const float* save_invstd, const float* gamma,
-                                float* dy, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                                int inner, int channels, void* workspace, size_t workspace_bytes, void* stream) {
-    AGCN_REQUIRE(mask_bits, AGCN_ERR_NULL, "agcn_bn_bwd_bits: null mask pointer");
-    return bn_bwd_impl(dout, nullptr, mask_bits, y, save_mean, save_invstd, gamma, dy, dgamma, dbeta, dres, dres_accumulate,
-                       1, inner, 0, channels, workspace, workspace_bytes, stream, 0, frozen_stats);
-}
-
-// agcn_bn_bwd_bits that also writes dy as bf16 pieces: dy_split [2][inner][channels] (see agcn_bn_apply_mask_split)
-extern "C" AGCN_API int agcn_bn_bwd_bits_split(const float* dout, const unsigned* mask_bits, const float* y,
-                                               const float* save_mean, const float* save_invstd, const float* gamma,
-                                               float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                                               int inner, int channels, void* workspace, size_t workspace_bytes, void* stream) {
-    AGCN_REQUIRE(mask_bits && dy && dy_split, AGCN_ERR_NULL, "agcn_bn_bwd_bits_split: null pointer");
-    return bn_bwd_impl(dout, nullptr, mask_bits, y, save_mean, save_invstd, gamma, dy, dgamma, dbeta, dres, dres_accumulate,
-                       1, inner, 0, channels, workspace, workspace_bytes, stream, 0, frozen_stats, static_cast<unsigned short*>(dy_split));
 }
 
 // Two BatchNorm backwards over the same masked upstream gradient in one pair of passes (see colsum_dual_kernel): BatchNorm A = (y_a,
@@ -929,23 +891,6 @@ extern "C" AGCN_API int agcn_bn_stats_partials(const float* x, int outer, int in
     return check_launch("agcn_bn_stats_partials");
 }
 
-// phase 1: dgamma / dbeta <- this rank's column sums (sum g xhat | sum g), nothing else is written.
-// phase 2: dy (dy_split, dres) from global_sums [2][C] = (sum g | sum g xhat) summed over all ranks and global_rows = the rows of all ranks.
-// mask_out / mask_bits / dy_split / pool_rows: the optional operands of agcn_bn_bwd, agcn_bn_bwd_bits(_split) and agcn_bn_bwd_pool.
-extern "C" AGCN_API int agcn_bn_bwd_sync(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
-                                         const float* save_mean, const float* save_invstd, const float* gamma,
-                                         float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
-                                         int outer, int inner, long long outer_stride, int channels, int pool_rows,
-                                         int phase, const float* global_sums, double global_rows,
-                                         void* workspace, size_t workspace_bytes, void* stream) {
-    AGCN_REQUIRE(phase == 1 || phase == 2, AGCN_ERR_UNSUPPORTED, "agcn_bn_bwd_sync: phase %d", phase);
-    AGCN_REQUIRE(phase == 2 || (dgamma && dbeta), AGCN_ERR_NULL, "agcn_bn_bwd_sync: phase 1 writes dgamma / dbeta");
-    AGCN_REQUIRE(pool_rows >= 0 && (pool_rows == 0 || (mask_bits && outer == 1 && inner % pool_rows == 0)), AGCN_ERR_BAD_SHAPE, "agcn_bn_bwd_sync: bad pooled shape");
-    return bn_bwd_impl(dout, mask_out, mask_bits, y, save_mean, save_invstd, gamma, dy, dgamma, dbeta, dres, dres_accumulate,
-                       outer, inner, outer_stride, channels, workspace, workspace_bytes, stream, pool_rows, 0,
-                       static_cast<unsigned short*>(dy_split), phase, global_sums, global_rows);
-}
-
 constexpr int kPoolParts = 8;
 
 extern "C" AGCN_API size_t agcn_bn_apply_pool_workspace_bytes(int groups, int channels) {
@@ -964,7 +909,7 @@ extern "C" AGCN_API int agcn_bn_apply_pool(const float* y, const float* scale, c
     RowMap m{1, groups * rows_per_group, 0, channels};
     AGCN_REQUIRE(agcn_bn_mask_words(1, groups * rows_per_group, channels) > 0 && channels % 32 == 0 &&
                  vec_ok(m, {y, scale, shift, res, scale2, shift2, pooled, workspace}),
-                 AGCN_ERR_UNSUPPORTED, "agcn_bn_apply_pool: layout not supported (use agcn_bn_apply_mask + agcn_pool_fwd)");
+                 AGCN_ERR_UNSUPPORTED, "agcn_bn_apply_pool: layout not supported (use agcn_bn_apply + agcn_pool_fwd)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     float* part = static_cast<float*>(workspace);
     const int cq = channels / 4;
@@ -975,17 +920,6 @@ extern "C" AGCN_API int agcn_bn_apply_pool(const float* y, const float* scale, c
     if (rc) return rc;
     pool_finalize_kernel<<<ceil_div((long long)groups * channels, 256), 256, 0, s>>>(part, pooled, kPoolParts, channels, groups, 1.f / (float)rows_per_group);
     return check_launch("agcn_bn_apply_pool(finalize)");
-}
-
-extern "C" AGCN_API int agcn_bn_bwd_pool(const float* dpooled, const unsigned* mask_bits, const float* y,
-                                         const float* save_mean, const float* save_invstd, const float* gamma,
-                                         float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
-                                         int groups, int rows_per_group, int channels, void* workspace, size_t workspace_bytes, void* stream) {
-    AGCN_REQUIRE(mask_bits && dpooled, AGCN_ERR_NULL, "agcn_bn_bwd_pool: null pointer");
-    AGCN_REQUIRE(groups > 0 && rows_per_group > 0, AGCN_ERR_BAD_SHAPE, "agcn_bn_bwd_pool: bad shape");
-    return bn_bwd_impl(dpooled, nullptr, mask_bits, y, save_mean, save_invstd, gamma, dy, dgamma, dbeta, dres, dres_accumulate,
-                       1, groups * rows_per_group, 0, channels, workspace, workspace_bytes, stream, rows_per_group, 0,
-                       static_cast<unsigned short*>(dy_split));
 }
 
 extern "C" AGCN_API int agcn_pool_fwd(const float* x, float* out, int groups, int rows_per_group, int channels, void* stream) {

@@ -26,7 +26,7 @@ long long launches() { return g_launches.load(std::memory_order_relaxed); }
 
 }  // namespace agcn
 
-extern "C" AGCN_API int agcn_version(void) { return 100; }
+extern "C" AGCN_API int agcn_version(void) { return 101; }
 
 extern "C" AGCN_API const char* agcn_last_error_string(void) { return agcn::error_buffer(); }
 

@@ -682,8 +682,8 @@ extern "C" AGCN_API size_t agcn_conv_wgrad_workspace_bytes(int nb, int t_in, int
 }
 
 // Weight gradient from operands that arrive split into bf16 pieces: dy_split [2][nb*t_out*v][cout] and x_split [2][nb*t_in*v][cin]
-// (plane 0 = h = bf16(value), plane 1 = m = bf16(value - h), round to nearest), as written by agcn_bn_apply_mask_split /
-// agcn_bn_bwd_bits_split.  Same arithmetic as the parity modes of agcn_conv_wgrad (h.h + h.m + m.h on kind::f16) without the
+// (plane 0 = h = bf16(value), plane 1 = m = bf16(value - h), round to nearest), as written by agcn_bn_apply /
+// agcn_bn_bwd (out_split / dy_split).  Same arithmetic as the parity modes of agcn_conv_wgrad (h.h + h.m + m.h on kind::f16) without the
 // in-kernel conversion.  No bias gradient.  AGCN_ERR_UNSUPPORTED (quiet) for channel counts that are not multiples of 64: use
 // agcn_conv_wgrad on the fp32 tensors then.
 extern "C" AGCN_API int agcn_conv_wgrad_presplit(const void* dy_split, const void* x_split, float* dw,

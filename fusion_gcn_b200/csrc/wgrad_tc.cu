@@ -42,7 +42,7 @@ struct WgArgs {
 // (second slot) -- MN-major 16-bit operands, 64 channels per 128-byte row, 8-row swizzle groups -- and the issuer runs
 // h.h + h.m + m.h on kind::f16 with K = 16 rows per MMA.  No lo ring: four 48 KB stages like the TF32 mode.
 // MODE 3: BF16x3 on operands that ARRIVE split -- [2][rows][C] bf16 tensors (plane 0 = h, plane 1 = m) written by the kernels that
-// produced the activations / gradients (agcn_bn_apply_mask_split, agcn_bn_bwd_bits_split).  One 5-D TMA box per operand lands as
+// produced the activations / gradients (agcn_bn_apply / agcn_bn_bwd with out_split / dy_split).  One 5-D TMA box per operand lands as
 // [64-channel block][piece][row][128 B], which IS the slot layout the issuer reads (h in the even slots, m in the odd ones): no
 // converter warps, no in-place rewrite -- the kernel is the TF32-mode pipeline with three bf16 MMAs per 16 rows.  In the in-kernel
 // conversion (MODE 2) the shared memory moves ~216 KB per 48 KB stage (TMA landing, conversion read + write, operand reads of three

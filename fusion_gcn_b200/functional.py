@@ -90,16 +90,6 @@ def _eval_affine(gamma, beta, buf: BnBuffers):
     return sc, sh
 
 
-def _apply(want_mask, *args, want_split=False, **kw):
-    """bn_apply -> (out, ReLU bit mask | None[, bf16 pieces of out | None]); the mask (and the pieces, the split operand of the weight
-    gradient of the convolution that consumes ``out``) are only produced when the backward will need them."""
-    if want_mask and want_split:
-        return K.bn_apply(*args, want_mask=True, want_split=True, **kw)
-    if want_mask:
-        return K.bn_apply(*args, want_mask=True, **kw)
-    return K.bn_apply(*args, **kw), None
-
-
 def _zero_bias(like, n):
     """Gradient of a conv bias that feeds a training-mode BatchNorm: BN subtracts the batch mean, so the loss does not
     depend on the bias and its gradient is identically zero (SURVEY D8; the reference's autograd produces ~1e-9 rounding
@@ -192,16 +182,13 @@ def gcn_forward(x, adj_a, adj_b, wa, ba, wb, bb, wd, bd, bn_w, bn_b, down_w, dow
     # the temporal convolution that follows takes its weight gradient from bf16 pieces of `o` written here, by the pass that
     # produces `o` anyway (agcn_conv_wgrad_presplit): no conversion pass in the weight-gradient kernel
     want_split = want_mask and spec.training and cout % 64 == 0 and prec != K.PREC_FP32_FFMA and prec != K.PREC_TF32
-    o_split = None
     if spec.has_down:
         yd, (sc2, sh2, mean2, invstd2) = _conv_bn(x, down_w.reshape(cout, 1, cin), down_b, dbn_w, dbn_b, spec.bn_down, spec.training, prec, sync=spec.sync)
-        r = _apply(want_mask, y, sc, sh, want_split=want_split, res_mode=K.RES_AFFINE, res=yd, scale2=sc2, shift2=sh2, relu=True)
+        o, o_bits, o_split = K.bn_apply(y, sc, sh, want_mask=want_mask, want_split=want_split, res_mode=K.RES_AFFINE, res=yd, scale2=sc2,
+                                        shift2=sh2, relu=True)
     else:
         yd = mean2 = invstd2 = None
-        r = _apply(want_mask, y, sc, sh, want_split=want_split, res_mode=K.RES_TENSOR, res=x, relu=True)
-    o, o_bits = r[0], r[1]
-    if len(r) == 3:
-        o_split = r[2]
+        o, o_bits, o_split = K.bn_apply(y, sc, sh, want_mask=want_mask, want_split=want_split, res_mode=K.RES_TENSOR, res=x, relu=True)
     if spec.attention_out is not None:
         spec.attention_out[:] = [p[:, k] for k in range(3)]
     if ctx is not None:
@@ -226,18 +213,12 @@ def gcn_backward(d_o, ctx, bn_w, dbn_w, down_w, spec: UnitSpec, dx=None, need_dx
     # eval mode with gradients (frozen-BN fine-tuning, saliency): the BatchNorms are affine maps of constants, and the biases of the
     # convolutions in front of them get real gradients (the column sums of dy) instead of the training mode's analytic zeros
     frozen = not spec.training
-    sk = dict(sync=spec.sync) if (spec.sync is not None and not frozen) else {}
     if z is None:
         z = K.joint_mix(x, g, width=cin, mode=K.MIX_AGG_FWD, precision=prec)
     if spec.has_down:
         # bn and down.1 both feed the ReLU of agcn.py:113-115: one pair of passes over the shared masked gradient for both backwards
-        both = None if sk else K.bn_bwd_dual(d_o, ctx["o_bits"], (y, ctx["mean"], ctx["invstd"], bn_w),
-                                             (ctx["yd"], ctx["mean2"], ctx["invstd2"], dbn_w), frozen=frozen)
-        if both is not None:
-            dy, dgam, dbet, _, dyd, dgam2, dbet2 = both
-        else:
-            dy, dgam, dbet = K.bn_bwd(d_o, o, y, ctx["mean"], ctx["invstd"], bn_w, mask_bits=ctx["o_bits"], frozen=frozen, **sk)
-            dyd, dgam2, dbet2 = K.bn_bwd(d_o, o, ctx["yd"], ctx["mean2"], ctx["invstd2"], dbn_w, mask_bits=ctx["o_bits"], frozen=frozen, **sk)
+        dy, dgam, dbet, _, dyd, dgam2, dbet2 = K.bn_bwd_dual(d_o, (y, ctx["mean"], ctx["invstd"], bn_w), (ctx["yd"], ctx["mean2"], ctx["invstd2"], dbn_w),
+                                                             mask_out=o, mask_bits=ctx["o_bits"], frozen=frozen, sync=spec.sync)
         wdown = down_w.reshape(cout, 1, cin)
         d_down_w, d_down_b = leaves.run(lambda: K.conv_wgrad(dyd, x, want_bias=frozen, precision=prec), dyd, x)
         if not frozen:
@@ -248,8 +229,8 @@ def gcn_backward(d_o, ctx, bn_w, dbn_w, down_w, spec: UnitSpec, dx=None, need_dx
     else:
         if need_dx and dx is None:
             dx = torch.empty_like(x)
-        dy, dgam, dbet = K.bn_bwd(d_o, o, y, ctx["mean"], ctx["invstd"], bn_w,
-                                  dres=dx if need_dx else None, dres_accumulate=have, mask_bits=ctx["o_bits"], frozen=frozen, **sk)
+        dy, dgam, dbet, _ = K.bn_bwd(d_o, o, y, ctx["mean"], ctx["invstd"], bn_w, dres=dx if need_dx else None, dres_accumulate=have,
+                                     mask_bits=ctx["o_bits"], frozen=frozen, sync=spec.sync)
         have = have or need_dx
         dgam2 = dbet2 = d_down_w = d_down_b = None
     dz = K.conv_fwd(dy, _t(ctx["wdc"]), precision=prec)                                # [nb,t,v,3*cin]
@@ -321,7 +302,7 @@ def tcn_forward(o, x_res, wt, bt, bn_w, bn_b, wr, br, rbn_w, rbn_b, spec: UnitSp
     pool = spec.pool_groups if (spec.pool_groups and spec.training and spec.relu_out and
                                 K.bn_pool_supported(u.numel() // u.shape[-1], u.shape[-1])) else 0
     apply = (lambda *a, **kw: K.bn_apply_pool(*a, groups=pool, **{k: v for k, v in kw.items() if k != "relu"})) if pool else \
-        (lambda *a, **kw: _apply(want_mask, *a, **kw))
+        (lambda *a, **kw: K.bn_apply(*a, want_mask=want_mask, **kw)[:2])
     if spec.residual == "identity":
         out, out_bits = apply(u, sc, sh, res_mode=K.RES_TENSOR, res=x_res, relu=spec.relu_out)
     elif spec.residual == "conv":
@@ -347,36 +328,21 @@ def tcn_backward(d_out, ctx, bn_w, rbn_w, spec: UnitSpec, need_dres=True, need_d
     ksz = spec.kernel_size
     mask = out if spec.relu_out else None
     bits = ctx["out_bits"] if spec.relu_out else None
-    pk = dict(pool_rows=ctx["pool_rows"]) if ctx.get("pool_rows") else {}       # d_out is then the pooled gradient [groups, c]
     d_xres = None
     d_wr = d_br = dgam2 = dbet2 = None
     frozen = not spec.training          # eval mode with gradients, see gcn_backward
-    pk["frozen"] = frozen
-    if spec.sync is not None and not frozen:
-        pk["sync"] = spec.sync
     # weight gradient of the temporal convolution from split operands: `o` as bf16 pieces from the gcn half's normalise pass, `du` as
     # bf16 pieces from the BatchNorm backward below (bit-mask forms only)
     o_split = ctx.get("o_split") if (not frozen and bits is not None) else None
-    du_split = None
-    if o_split is not None:
-        pk["want_split"] = True
+    # pool_rows > 0: d_out is the pooled gradient [groups, c]
+    kw = dict(mask_bits=bits, pool_rows=ctx.get("pool_rows", 0), frozen=frozen, sync=spec.sync, want_split=o_split is not None)
     if spec.residual == "identity":
         d_xres = torch.empty_like(x_res) if need_dres else None
-        du, dgam, dbet, *sp = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, dres=d_xres, dres_accumulate=False, mask_bits=bits, **pk)
-        du_split = sp[0] if sp else None
+        du, dgam, dbet, du_split = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, dres=d_xres, dres_accumulate=False, **kw)
     elif spec.residual == "conv":
         # the temporal BatchNorm and the residual branch's both feed the ReLU of agcn.py:135-136: one pair of passes for both backwards
-        both = None
-        if bits is not None and not pk.get("pool_rows") and "sync" not in pk:
-            both = K.bn_bwd_dual(d_out, bits, (u, ctx["t_mean"], ctx["t_invstd"], bn_w), (ctx["ur"], ctx["t_mean2"], ctx["t_invstd2"], rbn_w),
-                                 frozen=frozen, want_split=bool(pk.get("want_split")))
-        if both is not None:
-            du, dgam, dbet, du_split, dur, dgam2, dbet2 = both
-        else:
-            du, dgam, dbet, *sp = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, mask_bits=bits, **pk)
-            du_split = sp[0] if sp else None
-            pk.pop("want_split", None)
-            dur, dgam2, dbet2 = K.bn_bwd(d_out, mask, ctx["ur"], ctx["t_mean2"], ctx["t_invstd2"], rbn_w, mask_bits=bits, **pk)
+        du, dgam, dbet, du_split, dur, dgam2, dbet2 = K.bn_bwd_dual(d_out, (u, ctx["t_mean"], ctx["t_invstd"], bn_w),
+                                                                    (ctx["ur"], ctx["t_mean2"], ctx["t_invstd2"], rbn_w), mask_out=mask, **kw)
         d_wrp, d_br = leaves.run(lambda: K.conv_wgrad(dur, x_res, taps=1, stride=s, pad=0, want_bias=frozen, precision=prec), dur, x_res)
         if not frozen:
             d_br = _zero_bias(d_out, d_wrp.shape[0])
@@ -384,8 +350,7 @@ def tcn_backward(d_out, ctx, bn_w, rbn_w, spec: UnitSpec, need_dres=True, need_d
         if need_dres:
             d_xres = K.conv_fwd(dur, _t(ctx["wrp"]), t_out=x_res.shape[1], stride=s, pad=0, transposed=True, precision=prec)
     else:
-        du, dgam, dbet, *sp = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, mask_bits=bits, **pk)
-        du_split = sp[0] if sp else None
+        du, dgam, dbet, du_split = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, **kw)
     # the input gradient first (the gcn half's BatchNorm backward waits for it), then the weight gradient as a leaf beside that pass
     d_o = None
     if need_do:
@@ -570,9 +535,8 @@ class DataBnFn(torch.autograd.Function):
             sl = slice(mi * vc, (mi + 1) * vc)
             rowmap = (n, t, m * t * vc, vc)
             mean, invstd = ctx.saved[mi]
-            _, dg, db = K.bn_bwd(d_out[:, mi], None, x[:, mi], mean, invstd, gamma[sl], want_dy=need_dx,
-                                 dy=dx[:, mi] if need_dx else None, rowmap=rowmap, frozen=not ctx.training,
-                                 **(dict(sync=ctx.sync) if (ctx.sync is not None and ctx.training) else {}))
+            _, dg, db, _ = K.bn_bwd(d_out[:, mi], None, x[:, mi], mean, invstd, gamma[sl], want_dy=need_dx,
+                                    dy=dx[:, mi] if need_dx else None, rowmap=rowmap, frozen=not ctx.training, sync=ctx.sync)
             dgamma[sl] = dg
             dbeta[sl] = db
         return dx, dgamma, dbeta, None, None, None

@@ -109,12 +109,12 @@ class _RowBnFn(torch.autograd.Function):
                                              FN.BN_MOMENTUM, FN.BN_EPS, training)
         ctx.save_for_backward(x, gamma, mean, invstd)
         ctx.training = training
-        return FN.K.bn_apply(x, sc, sh)
+        return FN.K.bn_apply(x, sc, sh)[0]
 
     @staticmethod
     def backward(ctx, dy):
         x, gamma, mean, invstd = ctx.saved_tensors
-        dx, dgamma, dbeta = FN.K.bn_bwd(dy.contiguous(), None, x, mean, invstd, gamma, frozen=not ctx.training)
+        dx, dgamma, dbeta, _ = FN.K.bn_bwd(dy.contiguous(), None, x, mean, invstd, gamma, frozen=not ctx.training)
         return dx, dgamma, dbeta, None, None
 
 
@@ -125,7 +125,7 @@ class _AddReluFn(torch.autograd.Function):
     def forward(ctx, y, r):
         c = y.shape[-1]
         one, zero = torch.ones(c, device=y.device, dtype=y.dtype), torch.zeros(c, device=y.device, dtype=y.dtype)
-        out = FN.K.bn_apply(y, one, zero, res_mode=FN.K.RES_NONE if r is None else FN.K.RES_TENSOR, res=r, relu=True)
+        out = FN.K.bn_apply(y, one, zero, res_mode=FN.K.RES_NONE if r is None else FN.K.RES_TENSOR, res=r, relu=True)[0]
         ctx.save_for_backward(out)
         ctx.has_r = r is not None
         return out

@@ -403,127 +403,95 @@ def bn_stats_partials(x, rowmap=None):
 
 def bn_apply(y, scale, shift, *, res_mode=RES_NONE, res=None, scale2=None, shift2=None, relu=False, rowmap=None, out=None,
              want_mask=False, want_split=False):
-    """out = act(scale*y + shift + R).  ``want_mask``: also return the ReLU mask (out > 0) as one bit per element (int32 words,
-    agcn_bn_apply_mask) for bn_bwd(mask_bits=...), or None when the layout is not supported: -> (out, bits | None).
-    ``want_split`` (with want_mask): also return ``out`` as bf16 pieces [2, rows, c] for conv_wgrad_presplit (agcn_bn_apply_mask_split),
-    or None when the layout / channel count is not covered: -> (out, bits | None, split | None)."""
+    """out = act(scale*y + shift + R) -> (out, bits | None, split | None).  ``want_mask``: also the ReLU mask (out > 0) as one bit
+    per element (int32 words) for bn_bwd(mask_bits=...), None when the layout is not supported.  ``want_split`` (with want_mask):
+    also ``out`` as bf16 pieces [2, rows, c] for conv_wgrad_presplit, None when there is no bit mask or c is not a multiple of 64."""
     outer, inner, ostride, c = _rowmap(y, rowmap)
     if out is None:
         out = torch.empty_like(y)
     _check_strided(y, res, out)
     _check(scale, shift, scale2, shift2)
-    if want_mask:
-        words = capi.lib().agcn_bn_mask_words(outer, inner, c) if (y.is_contiguous() and out.is_contiguous() and (res is None or res.is_contiguous())) else 0
+    bits = split = None
+    if want_mask and y.is_contiguous() and out.is_contiguous() and (res is None or res.is_contiguous()):
+        words = capi.lib().agcn_bn_mask_words(outer, inner, c)
         if words:
             bits = torch.empty(words, device=y.device, dtype=torch.int32)
-            work = (0.0, 4.0 * outer * inner * c * (2 if res_mode == RES_NONE else 3))
             if want_split and c % 64 == 0:
                 split = torch.empty((2, inner, c), device=y.device, dtype=torch.bfloat16)
-                _call("agcn_bn_apply_mask_split", y.data_ptr(), _ptr(scale), _ptr(shift), res_mode, _ptr(res), _ptr(scale2), _ptr(shift2), int(relu),
-                      out.data_ptr(), bits.data_ptr(), split.data_ptr(), inner, c, _stream(), sig=(outer, inner, c, res_mode, int(relu), 1),
-                      work=(0.0, work[1] + 4.0 * inner * c), alias="agcn_bn_apply")
-                return out, bits, split
-            _call("agcn_bn_apply_mask", y.data_ptr(), _ptr(scale), _ptr(shift), res_mode, _ptr(res), _ptr(scale2), _ptr(shift2), int(relu),
-                  out.data_ptr(), bits.data_ptr(), inner, c, _stream(), sig=(outer, inner, c, res_mode, int(relu)),
-                  work=work, alias="agcn_bn_apply")
-            return (out, bits, None) if want_split else (out, bits)
     _call("agcn_bn_apply", y.data_ptr(), _ptr(scale), _ptr(shift), res_mode, _ptr(res), _ptr(scale2), _ptr(shift2), int(relu),
-          out.data_ptr(), outer, inner, ostride, c, _stream(), sig=(outer, inner, c, res_mode, int(relu)),
-          work=(0.0, 4.0 * outer * inner * c * (2 if res_mode == RES_NONE else 3)))
-    if want_mask:
-        return (out, None, None) if want_split else (out, None)
-    return out
+          out.data_ptr(), _ptr(bits), _ptr(split), outer, inner, ostride, c, _stream(),
+          sig=(outer, inner, c, res_mode, int(relu), int(bits is not None), int(split is not None)),
+          work=(0.0, 4.0 * outer * inner * c * (2 if res_mode == RES_NONE else 3) + (4.0 * inner * c if split is not None else 0.0)))
+    return out, bits, split
 
 
 def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy=None, dres=None, dres_accumulate=False,
            rowmap=None, mask_bits=None, pool_rows=0, frozen=False, want_split=False, sync=None):
-    """-> dy | None, dgamma, dbeta; optionally writes / accumulates the masked gradient into ``dres``.
-    ``sync`` (distributed.SyncBatchNorm, training mode only): the statistics were taken over all ranks, so the two column sums are
-    all-reduced between the sum pass and the apply pass (agcn_bn_bwd_sync); dgamma / dbeta stay this rank's own sums.
+    """-> (dy | None, dgamma, dbeta, dy_split | None); optionally writes / accumulates the masked gradient into ``dres``.
     ``dy`` may be a preallocated tensor addressed with the same rowmap as ``y``.  ``mask_bits`` (from bn_apply(want_mask=True))
-    replaces the fp32 tensor ``mask_out`` as the ReLU mask.  ``frozen``: the statistics are constants (eval-mode BatchNorm).
-    ``want_split``: -> dy, dgamma, dbeta, dy_split with dy also as bf16 pieces [2, rows, c] (agcn_bn_bwd_bits_split), or None in
-    the last place when the call is not the bit-mask form / the channel count is not a multiple of 64."""
+    replaces the fp32 tensor ``mask_out`` as the ReLU mask.  ``pool_rows`` > 0 (with mask_bits): ``dout`` is the gradient of the
+    fused mean pool, [groups, c], broadcast over the pool_rows rows of each group.  ``frozen``: the statistics are constants
+    (eval-mode BatchNorm).  ``want_split``: dy also as bf16 pieces [2, rows, c] for conv_wgrad_presplit, None when there is no bit
+    mask or c is not a multiple of 64.  ``sync`` (distributed.SyncBatchNorm, ignored when frozen): the statistics were taken over all
+    ranks, so the two column sums are all-reduced between the sum pass (phase 1) and the apply pass (phase 2); dgamma / dbeta stay
+    this rank's own sums."""
     outer, inner, ostride, c = _rowmap(y, rowmap)
     if want_dy and dy is None:
         dy = torch.empty_like(y)
     _check_strided(dout, mask_out, y, dy, dres)
     _check(save_mean, save_invstd, gamma)
-    dgb = torch.empty((2, c), device=y.device, dtype=torch.float32)
-    ws, nbytes = _bn_ws(c, y.device)
     if pool_rows and frozen:
         raise RuntimeError("bn_bwd: the pooled tail is a training-mode path")
-    if sync is not None and not frozen:
-        if mask_bits is not None:
-            if mask_bits.dtype != torch.int32 or not mask_bits.is_cuda:
-                raise RuntimeError("bn_bwd: mask_bits must be the int32 CUDA tensor returned by bn_apply(want_mask=True)")
-            _check(dout, y, dy, dres)
-        dy_split = torch.empty((2, inner, c), device=y.device, dtype=torch.bfloat16) if (want_split and dy is not None and mask_bits is not None
-                                                                                         and c % 64 == 0) else None
-        reads = 2 + (2.0 / 32 if mask_bits is not None else int(mask_out is not None))
-
-        def phase(k, sums, rows_all):
-            _call("agcn_bn_bwd_sync", dout.data_ptr(), _ptr(mask_out) if mask_bits is None else None, _ptr(mask_bits), y.data_ptr(),
-                  _ptr(save_mean), _ptr(save_invstd), _ptr(gamma), _ptr(dy), _ptr(dy_split), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres),
-                  int(dres_accumulate), outer, inner, ostride, c, int(pool_rows), k, _ptr(sums), float(rows_all), _ptr(ws), nbytes, _stream(),
-                  sig=(outer, inner, c, k, int(dy is not None), int(dres is not None), int(dres_accumulate), int(dy_split is not None)),
-                  work=(0.0, 4.0 * outer * inner * c * (reads if k == 1 else reads + int(dy is not None) * (1 + int(dy_split is not None))
-                                                       + int(dres is not None) * (1 + int(dres_accumulate)))), alias="agcn_bn_bwd")
-        phase(1, None, 0.0)
-        if dy is not None or dres is not None:
-            sums = sync.all_reduce(torch.stack([dgb[1], dgb[0]]))             # (sum g | sum g xhat) over all ranks
-            phase(2, sums, float(outer) * inner * sync.world)
-        return (dy, dgb[0], dgb[1], dy_split) if want_split else (dy, dgb[0], dgb[1])
-    if pool_rows:
-        # ``dout`` is the gradient of the fused mean pool, [groups, c], broadcast over the pool_rows rows of each group
-        _check(dout, y, dy, dres)
-        dy_split = torch.empty((2, inner, c), device=y.device, dtype=torch.bfloat16) if (want_split and dy is not None and c % 64 == 0) else None
-        _call("agcn_bn_bwd_pool", dout.data_ptr(), mask_bits.data_ptr(), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
-              _ptr(dy), _ptr(dy_split), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), dout.shape[0], int(pool_rows), c,
-              _ptr(ws), nbytes, _stream(), sig=(dout.shape[0], int(pool_rows), c, int(dy is not None), int(dres is not None)),
-              work=(0.0, 4.0 * inner * c * (2 + 2.0 / 32 + int(dy is not None) + int(dres is not None) * (1 + int(dres_accumulate)))),
-              alias="agcn_bn_bwd")
-        return (dy, dgb[0], dgb[1], dy_split) if want_split else (dy, dgb[0], dgb[1])
     if mask_bits is not None:
         if mask_bits.dtype != torch.int32 or not mask_bits.is_cuda:
             raise RuntimeError("bn_bwd: mask_bits must be the int32 CUDA tensor returned by bn_apply(want_mask=True)")
+        mask_out = None                 # the bits replace the tensor mask
+    if mask_bits is not None or pool_rows:
         _check(dout, y, dy, dres)
-        if want_split and dy is not None and c % 64 == 0:
-            dy_split = torch.empty((2, inner, c), device=y.device, dtype=torch.bfloat16)
-            _call("agcn_bn_bwd_bits_split", dout.data_ptr(), mask_bits.data_ptr(), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
-                  _ptr(dy), dy_split.data_ptr(), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), int(frozen), inner, c,
-                  _ptr(ws), nbytes, _stream(),
-                  sig=(outer, inner, c, 2, 1, int(dres is not None), int(dres_accumulate), 1),
-                  work=(0.0, 4.0 * outer * inner * c * (2 * 2 + 2.0 / 32 + 2 + int(dres is not None) * (1 + int(dres_accumulate)))),
-                  alias="agcn_bn_bwd")
-            return dy, dgb[0], dgb[1], dy_split
-        _call("agcn_bn_bwd_bits", dout.data_ptr(), mask_bits.data_ptr(), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
-              _ptr(dy), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), int(frozen), inner, c, _ptr(ws), nbytes, _stream(),
-              sig=(outer, inner, c, 2, int(dy is not None), int(dres is not None), int(dres_accumulate)),
-              work=(0.0, 4.0 * outer * inner * c * (2 * 2 + 2.0 / 32 + int(dy is not None) + int(dres is not None) * (1 + int(dres_accumulate)))),
-              alias="agcn_bn_bwd")
-        return (dy, dgb[0], dgb[1], None) if want_split else (dy, dgb[0], dgb[1])
-    _call("agcn_bn_bwd", dout.data_ptr(), _ptr(mask_out), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
-          _ptr(dy), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), int(frozen), outer, inner, ostride, c,
-          _ptr(ws), nbytes, _stream(),
-          sig=(outer, inner, c, int(mask_out is not None), int(dy is not None), int(dres is not None), int(dres_accumulate)),
-          # two passes over (dout, y[, mask]); the second writes dy [and dres, read first when accumulating]
-          work=(0.0, 4.0 * outer * inner * c * (2 * (2 + int(mask_out is not None)) + int(dy is not None)
-                                               + int(dres is not None) * (1 + int(dres_accumulate)))))
-    return (dy, dgb[0], dgb[1], None) if want_split else (dy, dgb[0], dgb[1])
+    dy_split = torch.empty((2, inner, c), device=y.device, dtype=torch.bfloat16) if (want_split and dy is not None and mask_bits is not None
+                                                                                     and c % 64 == 0) else None
+    dgb = torch.empty((2, c), device=y.device, dtype=torch.float32)
+    ws, nbytes = _bn_ws(c, y.device)
+    mask_kind = 2 if mask_bits is not None else int(mask_out is not None)
+    writes = int(dy is not None) + int(dres is not None) * (1 + int(dres_accumulate))
+    pieces = int(dy_split is not None)
+
+    def run(phase, planes, sums=None, rows_all=0.0):
+        # planes: the algorithmic bytes of the call in fp32 planes of y
+        _call("agcn_bn_bwd", dout.data_ptr(), _ptr(mask_out), _ptr(mask_bits), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
+              _ptr(dy), _ptr(dy_split), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), int(frozen),
+              outer, inner, ostride, c, int(pool_rows), phase, _ptr(sums), float(rows_all), _ptr(ws), nbytes, _stream(),
+              sig=(outer, inner, c, mask_kind, int(pool_rows), phase, int(dy is not None), int(dres is not None), int(dres_accumulate), pieces),
+              work=(0.0, 4.0 * outer * inner * c * planes))
+
+    if sync is not None and not frozen:
+        reads = 2 + (2.0 / 32 if mask_bits is not None else int(mask_out is not None))
+        run(1, reads)
+        if dy is not None or dres is not None:
+            sums = sync.all_reduce(torch.stack([dgb[1], dgb[0]]))             # (sum g | sum g xhat) over all ranks
+            run(2, reads + writes + pieces, sums, float(outer) * inner * sync.world)
+    elif pool_rows:
+        run(0, 2 + 2.0 / 32 + writes)                 # y and the bits in both passes; the pooled gradient is negligible
+    else:
+        # two passes over (dout, y[, mask]); the second writes dy [and its pieces, and dres, read first when accumulating]
+        run(0, 2 * (2 + (1.0 / 32 if mask_bits is not None else int(mask_out is not None))) + writes + pieces)
+    return dy, dgb[0], dgb[1], dy_split
 
 
-def bn_bwd_dual(dout, mask_bits, a, b, *, frozen=False, want_split=False):
-    """Two BatchNorm backwards that share the masked upstream gradient (agcn_bn_bwd_bits_dual): ``a`` / ``b`` = (y, save_mean,
-    save_invstd, gamma) of the two BatchNorms.  -> (dy_a, dgamma_a, dbeta_a, dy_a_split | None, dy_b, dgamma_b, dbeta_b), or None
-    when the layout is not covered (no bit mask) -- call bn_bwd twice then."""
+def bn_bwd_dual(dout, a, b, *, mask_out=None, mask_bits=None, frozen=False, want_split=False, pool_rows=0, sync=None):
+    """Two BatchNorm backwards over the same upstream gradient and ReLU mask: ``a`` / ``b`` = (y, save_mean, save_invstd, gamma) of
+    the two BatchNorms.  -> (dy_a, dgamma_a, dbeta_a, dy_a_split | None, dy_b, dgamma_b, dbeta_b); only BatchNorm A gets bf16 pieces.
+    Where agcn_bn_bwd_bits_dual covers the call (bit mask, no pooled gradient, no synchronised statistics, contiguous tensors) the
+    masked gradient is read once per pass for both; otherwise this is two bn_bwd calls."""
     ya, mean_a, invstd_a, gamma_a = a
     yb, mean_b, invstd_b, gamma_b = b
     c = ya.shape[-1]
     inner = ya.numel() // c
-    if mask_bits is None or not ya.is_contiguous() or not yb.is_contiguous() or not dout.is_contiguous() or tuple(ya.shape) != tuple(yb.shape) \
-            or tuple(dout.shape) != tuple(ya.shape) or capi.lib().agcn_bn_mask_words(1, inner, c) == 0:
-        return None
+    if mask_bits is None or pool_rows or (sync is not None and not frozen) or not ya.is_contiguous() or not yb.is_contiguous() \
+            or not dout.is_contiguous() or tuple(ya.shape) != tuple(yb.shape) or tuple(dout.shape) != tuple(ya.shape) \
+            or capi.lib().agcn_bn_mask_words(1, inner, c) == 0:
+        kw = dict(mask_bits=mask_bits, frozen=frozen, pool_rows=pool_rows, sync=sync)
+        return bn_bwd(dout, mask_out, *a, want_split=want_split, **kw) + bn_bwd(dout, mask_out, *b, **kw)[:3]
     _check(dout, ya, yb, mean_a, invstd_a, gamma_a, mean_b, invstd_b, gamma_b)
     dya, dyb = torch.empty_like(ya), torch.empty_like(yb)
     split = torch.empty((2, inner, c), device=ya.device, dtype=torch.bfloat16) if (want_split and c % 64 == 0) else None
@@ -539,7 +507,7 @@ def bn_bwd_dual(dout, mask_bits, a, b, *, frozen=False, want_split=False):
 
 
 def bn_pool_supported(rows: int, channels: int) -> bool:
-    """Whether the fused BN-apply + mean-pool tail (agcn_bn_apply_pool / agcn_bn_bwd_pool) covers this layout."""
+    """Whether the fused BN-apply + mean-pool tail (agcn_bn_apply_pool, and bn_bwd with pool_rows) covers this layout."""
     return channels % 32 == 0 and capi.lib().agcn_bn_mask_words(1, rows, channels) > 0
 
 

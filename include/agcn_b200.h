@@ -122,7 +122,7 @@ int agcn_conv_wgrad(const float* dy, const float* x, float* dw, float* dbias,
 
 /* The same weight gradient (no bias gradient) from operands that ARRIVE split into the bf16 pieces the
  * parity modes multiply: dy_split [2][nb*t_out*v][cout], x_split [2][nb*t_in*v][cin] bf16, plane 0 = h = bf16(value), plane 1 =
- * m = bf16(value - h) -- written by agcn_bn_apply_mask_split / agcn_bn_bwd_bits_split, the kernels that produce the activations
+ * m = bf16(value - h) -- written by agcn_bn_apply / agcn_bn_bwd (out_split / dy_split), the kernels that produce the activations
  * and their gradients anyway.  The in-kernel conversion of agcn_conv_wgrad is what bounds it (shared-memory bandwidth); without
  * it the kernel runs at the tensor rate of three bf16 MMAs.  Same workspace as agcn_conv_wgrad.  Returns AGCN_ERR_UNSUPPORTED
  * (no error string) unless cin and cout are multiples of 64.                                                                   */
@@ -198,48 +198,45 @@ int agcn_bn_finalize(const float* part, int nparts, long long rows, int channels
                      float* scale, float* shift, float* save_mean, float* save_invstd, void* stream);
 
 /* out = act(scale*y + shift + R),  R = 0 | res | scale2*res + shift2;  act = ReLU when relu!=0.
- * (agcn.py:113-115 and :135-136).  Same addressing as agcn_bn_stats for y / res / out.                   */
+ * (agcn.py:113-115 and :135-136).  Same addressing as agcn_bn_stats for y / res / out.
+ * Two optional outputs (NULL: not written) for the backward:
+ *   mask_bits: the ReLU mask (out > 0) as ONE BIT per element, bit e & 31 of word e >> 5, e = row * channels + c, for
+ *     agcn_bn_bwd (its two passes then read 1/32 of the mask bytes).  Needs agcn_bn_mask_words(outer, inner, channels) > 0.
+ *   out_split: `out` once more as the bf16 pieces the parity modes multiply, [2][inner][channels] bf16, plane 0 = h = bf16(out),
+ *     plane 1 = m = bf16(out - h) -- the operand format of agcn_conv_wgrad_presplit.  One more plane written by a kernel that
+ *     streams the tensor anyway, instead of a conversion pass in shared memory for every tile of the weight gradient.
+ *     Needs outer == 1 and a vectorisable layout.
+ * An optional output the layout does not support is AGCN_ERR_UNSUPPORTED.                                                */
 int agcn_bn_apply(const float* y, const float* scale, const float* shift,
                   int res_mode, const float* res, const float* scale2, const float* shift2,
-                  int relu, float* out, int outer, int inner, long long outer_stride, int channels, void* stream);
+                  int relu, float* out, unsigned* mask_bits, void* out_split,
+                  int outer, int inner, long long outer_stride, int channels, void* stream);
 
-/* ReLU mask as ONE BIT per element (bit e & 31 of word e >> 5, e = row * channels + c) for contiguous [inner][channels]
- * tensors: agcn_bn_apply_mask = agcn_bn_apply that also writes the bits of (out > 0); agcn_bn_bwd_bits = agcn_bn_bwd reading
- * them instead of the fp32 tensor mask_out (the two backward passes then read 1/32 of the mask bytes).
- * agcn_bn_mask_words returns the number of 32-bit words, or 0 when the layout is not supported (outer != 1, channels
- * not a multiple of 4, channels/4 not a divisor of 256) -- use the tensor mask then.                                  */
+/* Number of 32-bit words of the bit mask of agcn_bn_apply, or 0 when the layout is not supported (outer != 1, channels not a
+ * multiple of 4, channels/4 not a divisor of 256) -- use the fp32 tensor as the mask then.                              */
 size_t agcn_bn_mask_words(int outer, int inner, int channels);
-int agcn_bn_apply_mask(const float* y, const float* scale, const float* shift,
-                       int res_mode, const float* res, const float* scale2, const float* shift2,
-                       int relu, float* out, unsigned* mask_bits, int inner, int channels, void* stream);
-int agcn_bn_bwd_bits(const float* dout, const unsigned* mask_bits, const float* y,
-                     const float* save_mean, const float* save_invstd, const float* gamma,
-                     float* dy, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                     int inner, int channels, void* workspace, size_t workspace_bytes, void* stream);
-
-/* agcn_bn_apply_mask / agcn_bn_bwd_bits that ALSO leave their fp32 output (out / dy) as the bf16 pieces the parity modes multiply:
- * [2][inner][channels] bf16, plane 0 = h = bf16(value), plane 1 = m = bf16(value - h) -- the operand format of
- * agcn_conv_wgrad_presplit.  One more plane written by kernels that stream the tensor anyway, instead of a conversion pass in
- * shared memory for every tile of the weight gradient.  Same layout restrictions as the bit-mask variants.               */
-int agcn_bn_apply_mask_split(const float* y, const float* scale, const float* shift,
-                             int res_mode, const float* res, const float* scale2, const float* shift2,
-                             int relu, float* out, unsigned* mask_bits, void* out_split, int inner, int channels, void* stream);
-int agcn_bn_bwd_bits_split(const float* dout, const unsigned* mask_bits, const float* y,
-                           const float* save_mean, const float* save_invstd, const float* gamma,
-                           float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                           int inner, int channels, void* workspace, size_t workspace_bytes, void* stream);
 
 /* BatchNorm backward through an optional ReLU mask:
- *   g = dout * [mask_out > 0]  (g = dout when mask_out == NULL)
+ *   g = dout * [mask > 0]  (g = dout without a mask)
  *   dbeta = sum g;  dgamma = sum g*xhat;  dy = gamma*invstd*(g - dbeta/m - xhat*dgamma/m),  xhat = (y-mean)*invstd
+ * The mask is the fp32 tensor mask_out (addressed like y) or the bits of agcn_bn_apply (mask_bits), never both; both NULL: no mask.
  * If dres != NULL the masked gradient g is also written (dres_accumulate==0) or added to dres
  * (gradient of an identity residual / of the tensor R above).  dy may be NULL (only sums wanted).
+ * dy_split (NULL: not written; needs dy): dy once more as bf16 pieces, layout and restrictions of agcn_bn_apply's out_split.
  * frozen_stats != 0: mean / invstd are constants -- the backward of an eval-mode BatchNorm on its running statistics (the
- * reference's autograd under model.eval()): dy = gamma*invstd*g, dgamma and dbeta as above.                                  */
-int agcn_bn_bwd(const float* dout, const float* mask_out, const float* y,
+ *   reference's autograd under model.eval()): dy = gamma*invstd*g, dgamma and dbeta as above.  Only with pool_rows == 0 and phase 0.
+ * pool_rows > 0 (with mask_bits, outer == 1): dout is the pooled gradient of agcn_bn_apply_pool, [inner / pool_rows][channels],
+ *   broadcast over its group: dout[row][c] = dpooled[row / pool_rows][c] / pool_rows.
+ * phase 0: the whole backward.  Phases 1 and 2 are the two halves of a synchronised BatchNorm, either side of the caller's
+ *   all-reduce: phase 1 writes only dgamma / dbeta = this rank's sums (sum g xhat | sum g); phase 2 writes dy (dy_split, dres) from
+ *   global_sums [2][channels] = (sum g | sum g xhat) all-reduced over the ranks and global_rows = the rows of all ranks.
+ *   global_sums / global_rows are read in phase 2 only.
+ * workspace: agcn_bn_workspace_bytes(channels).                                                                              */
+int agcn_bn_bwd(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
                 const float* save_mean, const float* save_invstd, const float* gamma,
-                float* dy, float* dgamma, float* dbeta, float* dres, int dres_accumulate, int frozen_stats,
-                int outer, int inner, long long outer_stride, int channels,
+                float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
+                int frozen_stats, int outer, int inner, long long outer_stride, int channels, int pool_rows,
+                int phase, const float* global_sums, double global_rows,
                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- pooling (agcn.py:194-196): out[g][c] = mean over rows_per_group rows of x[g][row][c] ------------ */
@@ -249,25 +246,19 @@ int agcn_pool_bwd(const float* dout, float* dx, int groups, int rows_per_group, 
 /* Fused tail of the model: the last unit's out = relu(scale*y + shift + R) (agcn.py:135-136) feeds only the global mean pool
  * x.view(N, M, C, -1).mean(3).mean(1) (agcn.py:194-196), so `out` is never written: agcn_bn_apply_pool leaves the pooled means
  * pooled[groups][channels] (group g = rows [g*rows_per_group, (g+1)*rows_per_group)) and the ReLU mask bits (layout of
- * agcn_bn_apply_mask); agcn_bn_bwd_pool is agcn_bn_bwd_bits whose upstream gradient is the pooled gradient broadcast over the
- * group (dout[row][c] = dpooled[row / rows_per_group][c] / rows_per_group).  channels must be a multiple of 32 with
+ * agcn_bn_apply); its backward is agcn_bn_bwd with pool_rows = rows_per_group.  channels must be a multiple of 32 with
  * agcn_bn_mask_words(1, groups*rows_per_group, channels) > 0, else AGCN_ERR_UNSUPPORTED (use the unfused calls).                  */
 size_t agcn_bn_apply_pool_workspace_bytes(int groups, int channels);
 int agcn_bn_apply_pool(const float* y, const float* scale, const float* shift,
                        int res_mode, const float* res, const float* scale2, const float* shift2,
                        unsigned* mask_bits, float* pooled, int groups, int rows_per_group, int channels,
                        void* workspace, size_t workspace_bytes, void* stream);
-int agcn_bn_bwd_pool(const float* dpooled, const unsigned* mask_bits, const float* y,
-                     const float* save_mean, const float* save_invstd, const float* gamma,
-                     float* dy, void* dy_split /* NULL, or dy once more as bf16 pieces, see agcn_bn_bwd_bits_split */,
-                     float* dgamma, float* dbeta, float* dres, int dres_accumulate,
-                     int groups, int rows_per_group, int channels, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Two BatchNorm backwards over the SAME masked upstream gradient in one pair of passes: the gcn half's bn and down.1 both feed the
  * ReLU of agcn.py:113-115, the temporal BatchNorm and the residual branch's both feed the one of agcn.py:135-136, so g = dout * mask
  * is read once per pass for both (8 plane passes instead of 10).  BatchNorm A may also leave dy_a as bf16 pieces (dy_a_split, see
- * agcn_bn_bwd_bits_split).  workspace: 2 x agcn_bn_workspace_bytes(channels).  Returns AGCN_ERR_UNSUPPORTED (no error string) for
- * layouts without a bit mask (agcn_bn_mask_words == 0): call agcn_bn_bwd_bits twice then.                                        */
+ * agcn_bn_bwd).  workspace: 2 x agcn_bn_workspace_bytes(channels).  Returns AGCN_ERR_UNSUPPORTED (no error string) for
+ * layouts without a bit mask (agcn_bn_mask_words == 0): call agcn_bn_bwd twice then.                                             */
 int agcn_bn_bwd_bits_dual(const float* dout, const unsigned* mask_bits,
                           const float* y_a, const float* mean_a, const float* invstd_a, const float* gamma_a,
                           float* dy_a, void* dy_a_split, float* dgamma_a, float* dbeta_a,
@@ -280,19 +271,10 @@ int agcn_bn_bwd_bits_dual(const float* dout, const unsigned* mask_bits,
  * statistics are taken over all ranks).  The collectives stay with the caller; the library provides the halves either side of them.
  * agcn_bn_stats_partials: part [nparts][4][channels] = per row partition the shifted sum | shifted sum of squares | pivot | row count
  * of x -- the layout agcn_conv_fwd_stats writes and agcn_bn_finalize merges, so the partials of all ranks are concatenated
- * (all-gather) and finalised with rows = the global row count.  agcn_bn_bwd_sync phase 1: dgamma / dbeta <- this rank's sums
- * (sum g xhat | sum g; nothing else written); phase 2: dy (dy_split, dres) from global_sums [2][channels] = (sum g | sum g xhat)
- * all-reduced over the ranks and global_rows.  mask_out / mask_bits / dy_split / pool_rows are the optional operands of agcn_bn_bwd,
- * agcn_bn_bwd_bits(_split) and agcn_bn_bwd_pool (pool_rows > 0: dout is the pooled gradient [inner / pool_rows][channels]).   */
+ * (all-gather) and finalised with rows = the global row count.  The backward halves are agcn_bn_bwd phases 1 and 2.             */
 size_t agcn_bn_stats_partials_bytes(int channels);
 int agcn_bn_stats_partials(const float* x, int outer, int inner, long long outer_stride, int channels,
                            float* part, size_t part_bytes, int* nparts, void* workspace, size_t workspace_bytes, void* stream);
-int agcn_bn_bwd_sync(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
-                     const float* save_mean, const float* save_invstd, const float* gamma,
-                     float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
-                     int outer, int inner, long long outer_stride, int channels, int pool_rows,
-                     int phase, const float* global_sums, double global_rows,
-                     void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- classifier head fused with its loss -------------------------------------------------------------
  * logits = x . w^T + bias (nn.Linear, agcn.py:178,198-199) and loss = mean_n( logsumexp(logits[n]) - logits[n][label[n]] )

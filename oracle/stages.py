@@ -249,9 +249,9 @@ def conv_wgrad_presplit(dy_split, x_split, shape, *, taps=1, stride=1, pad=0):
 def bn_apply(y, scale, shift, *, res_mode=RES_NONE, res=None, scale2=None, shift2=None, relu=False, rowmap=None, out=None,
              want_mask=False, want_split=False):
     r = _bn_apply(y, scale, shift, res_mode=res_mode, res=res, scale2=scale2, shift2=shift2, relu=relu, rowmap=rowmap, out=out)
-    if want_mask and want_split:
-        return r, (r > 0), (bf16_split(r) if r.shape[-1] % 64 == 0 and rowmap is None else None)
-    return (r, (r > 0)) if want_mask else r            # the "bit mask" of the CUDA path is a bool tensor here
+    bits = (r > 0) if want_mask else None              # the "bit mask" of the CUDA path is a bool tensor here
+    split = bf16_split(r) if (want_mask and want_split and r.shape[-1] % 64 == 0 and rowmap is None) else None
+    return r, bits, split
 
 
 def _bn_apply(y, scale, shift, *, res_mode=RES_NONE, res=None, scale2=None, shift2=None, relu=False, rowmap=None, out=None):
@@ -271,11 +271,6 @@ def _bn_apply(y, scale, shift, *, res_mode=RES_NONE, res=None, scale2=None, shif
 
 def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy=None, dres=None, dres_accumulate=False,
            rowmap=None, mask_bits=None, pool_rows=0, frozen=False, want_split=False, sync=None):
-    if want_split:
-        dy, dgamma, dbeta = bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, want_dy=want_dy, dy=dy, dres=dres, dres_accumulate=dres_accumulate,
-                                   rowmap=rowmap, mask_bits=mask_bits, pool_rows=pool_rows, frozen=frozen, sync=sync)
-        ok = dy is not None and mask_bits is not None and rowmap is None and dy.shape[-1] % 64 == 0
-        return dy, dgamma, dbeta, (bf16_split(dy) if ok else None)
     if pool_rows:          # dout is the pooled gradient [groups, c]: broadcast over the rows of each group, divided by their number
         groups, c = dout.shape
         dout = (dout / pool_rows).reshape(groups, 1, c).expand(groups, pool_rows, c).reshape(y.shape).contiguous()
@@ -293,7 +288,7 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
     dgamma = (g * xhat).sum(dim=red)
     s1, s2 = dbeta, dgamma
     if sync is not None and not frozen:
-        # synchronised BatchNorm (agcn_bn_bwd_sync): the two sums and the row count over all ranks; dgamma / dbeta stay this rank's own
+        # synchronised BatchNorm (agcn_bn_bwd phases 1 and 2): the two sums and the row count over all ranks; dgamma / dbeta stay this rank's own
         both = sync.all_reduce(torch.stack([dbeta, dgamma]))
         s1, s2, m = both[0], both[1], m * sync.world
     if want_dy:
@@ -308,16 +303,15 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
             dv += g
         else:
             dv.copy_(g)
-    return dy, dgamma, dbeta
+    ok = want_split and dy is not None and mask_bits is not None and rowmap is None and dy.shape[-1] % 64 == 0
+    return dy, dgamma, dbeta, (bf16_split(dy) if ok else None)
 
 
-def bn_bwd_dual(dout, mask_bits, a, b, *, frozen=False, want_split=False):
-    """agcn_bn_bwd_bits_dual: two BatchNorm backwards over the same masked upstream gradient (None when there is no bit mask)."""
-    if mask_bits is None:
-        return None
-    dya, dga, dba, *sp = bn_bwd(dout, None, a[0], a[1], a[2], a[3], mask_bits=mask_bits, frozen=frozen, want_split=want_split)
-    dyb, dgb_, dbb = bn_bwd(dout, None, b[0], b[1], b[2], b[3], mask_bits=mask_bits, frozen=frozen)
-    return dya, dga, dba, (sp[0] if sp else None), dyb, dgb_, dbb
+def bn_bwd_dual(dout, a, b, *, mask_out=None, mask_bits=None, frozen=False, want_split=False, pool_rows=0, sync=None):
+    """Two BatchNorm backwards over the same upstream gradient and ReLU mask (agcn_bn_bwd_bits_dual, or two bn_bwd calls); only
+    BatchNorm A gets bf16 pieces."""
+    kw = dict(mask_bits=mask_bits, frozen=frozen, pool_rows=pool_rows, sync=sync)
+    return bn_bwd(dout, mask_out, *a, want_split=want_split, **kw) + bn_bwd(dout, mask_out, *b, **kw)[:3]
 
 
 def bn_pool_supported(rows, channels):

@@ -46,3 +46,24 @@ def test_argument_validation_without_gpu():
     assert rc == 1
     with pytest.raises(RuntimeError, match="status 1"):
         capi.check(rc, "agcn_conv_fwd")
+
+
+@pytest.mark.parametrize("operands,status,message", [
+    (dict(frozen=1, pool_rows=4, mask_bits=1), 2, b"frozen statistics"),
+    (dict(frozen=1, phase=1), 2, b"frozen statistics"),
+    (dict(frozen=1, phase=2), 2, b"frozen statistics"),
+    (dict(phase=3), 2, b"phase 3"),
+    (dict(phase=-1), 2, b"phase -1"),
+    (dict(mask_out=1, mask_bits=1), 2, b"mask_out and mask_bits"),
+    (dict(dy=None, dy_split=1), 6, b"dy_split needs dy"),
+])
+def test_batchnorm_backward_rejects_contradictory_operands(operands, status, message):
+    """agcn_bn_bwd refuses operand combinations that no form of the backward covers before it launches anything (the workspace is
+    NULL, so a call that got past these checks would stop at the null-pointer check instead of reaching the device)."""
+    from fusion_gcn_b200 import capi
+    lib = capi.lib()
+    a = dict(mask_out=None, mask_bits=None, dy=1, dy_split=None, frozen=0, pool_rows=0, phase=0)
+    a.update(operands)
+    rc = lib.agcn_bn_bwd(1, a["mask_out"], a["mask_bits"], 1, 1, 1, 1, a["dy"], a["dy_split"], 1, 1, None, 0, a["frozen"],
+                         1, 64, 0, 64, a["pool_rows"], a["phase"], 1, 64.0, None, 0, None)
+    assert rc == status and message in lib.agcn_last_error_string()

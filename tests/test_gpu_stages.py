@@ -70,14 +70,15 @@ def test_conv_fwd_dgrad_wgrad(K, nb, t_in, v, cin, cout, taps, stride, mode):
 
 
 @pytest.mark.parametrize("rows,c", [(1000, 64), (4099, 256), (777, 128), (333, 192), (50, 32)])
-def test_batchnorm_kernels_also_write_bf16_pieces(K, rows, c):
-    """agcn_bn_apply_mask_split / agcn_bn_bwd_bits_split: the fp32 results are those of the plain bit-mask calls bit for bit, the extra
-    output is their (h, m) bf16 split -- the operand format of agcn_conv_wgrad_presplit; channel counts that are not a multiple of 64
-    return None in its place."""
+def test_bn_apply_and_bn_bwd_bf16_pieces_are_optional_outputs(K, rows, c):
+    """agcn_bn_apply / agcn_bn_bwd with their bf16-pieces output (out_split / dy_split): the fp32 results are those of the same calls
+    without it bit for bit, the extra output is their (h, m) bf16 split -- the operand format of agcn_conv_wgrad_presplit; channel
+    counts that are not a multiple of 64 return None in its place."""
     y, res = rnd(rows, c).cuda(), rnd(rows, c, seed=1).cuda()
     sc, sh = (rnd(c, seed=2) * 0.3 + 1).cuda(), (rnd(c, seed=3) * 0.1).cuda()
-    o0, b0 = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
+    o0, b0, sp0 = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
     o1, b1, sp = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True, want_split=True)
+    assert sp0 is None
     assert torch.equal(o0, o1)
     if b0 is None:                       # (192 channels: no bit-mask layout, hence no fused pieces either)
         assert b1 is None and sp is None
@@ -87,7 +88,8 @@ def test_batchnorm_kernels_also_write_bf16_pieces(K, rows, c):
     mean, invstd, gamma = (rnd(c, seed=5) * 0.1).cuda(), (rnd(c, seed=6).abs() + 0.5).cuda(), (rnd(c, seed=7) * 0.3 + 1).cuda()
     d0 = K.bn_bwd(dout, None, y, mean, invstd, gamma, mask_bits=b0)
     d1 = K.bn_bwd(dout, None, y, mean, invstd, gamma, mask_bits=b0, want_split=True)
-    assert all(torch.equal(a, b) for a, b in zip(d0, d1[:3]))
+    assert d0[3] is None
+    assert all(torch.equal(a, b) for a, b in zip(d0[:3], d1[:3]))
     if c % 64:
         assert sp is None and d1[3] is None
         return
@@ -96,22 +98,23 @@ def test_batchnorm_kernels_also_write_bf16_pieces(K, rows, c):
 
 
 @pytest.mark.parametrize("rows,c,frozen", [(1000, 64, False), (4099, 256, False), (777, 128, True), (333, 192, False), (120000, 128, False)])
-def test_two_batchnorm_backwards_over_one_upstream_gradient(K, rows, c, frozen):
-    """agcn_bn_bwd_bits_dual (bn + down.1 of the gcn half, the temporal + residual BatchNorms of the unit): same sums in the same order
-    and the same apply formula as two agcn_bn_bwd_bits calls; layouts without a bit mask return None."""
+def test_bn_bwd_dual_matches_two_bn_bwd_calls(K, rows, c, frozen):
+    """bn_bwd_dual on agcn_bn_bwd_bits_dual (bn + down.1 of the gcn half, the temporal + residual BatchNorms of the unit): same sums in
+    the same order and the same apply formula as two agcn_bn_bwd calls; layouts without a bit mask make exactly those two calls."""
     ya, yb, res = rnd(rows, c).cuda(), rnd(rows, c, seed=9).cuda(), rnd(rows, c, seed=1).cuda()
     sc, sh = (rnd(c, seed=2) * 0.3 + 1).cuda(), (rnd(c, seed=3) * 0.1).cuda()
-    _, bits = K.bn_apply(ya, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
+    out, bits, _ = K.bn_apply(ya, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
     dout = rnd(rows, c, seed=4).cuda()
     stats = [((rnd(c, seed=5 + i) * 0.1).cuda(), (rnd(c, seed=7 + i).abs() + 0.5).cuda(), (rnd(c, seed=11 + i) * 0.3 + 1).cuda()) for i in range(2)]
     a, b = (ya, *stats[0]), (yb, *stats[1])
-    got = K.bn_bwd_dual(dout, bits, a, b, frozen=frozen, want_split=True)
+    got = K.bn_bwd_dual(dout, a, b, mask_out=out, mask_bits=bits, frozen=frozen, want_split=True)
+    wa = K.bn_bwd(dout, out, ya, *stats[0], mask_bits=bits, frozen=frozen, want_split=True)
+    wb = K.bn_bwd(dout, out, yb, *stats[1], mask_bits=bits, frozen=frozen)
     if bits is None:
-        assert got is None
+        assert got[3] is None and wa[3] is None
+        assert all(torch.equal(g, w) for g, w in zip(got[:3] + got[4:], wa[:3] + wb[:3]))
         return
-    wa = K.bn_bwd(dout, None, ya, *stats[0], mask_bits=bits, frozen=frozen, want_split=True)
-    wb = K.bn_bwd(dout, None, yb, *stats[1], mask_bits=bits, frozen=frozen)
-    for g, w in zip(got[:3] + got[4:], wa[:3] + wb):
+    for g, w in zip(got[:3] + got[4:], wa[:3] + wb[:3]):
         assert rel_err(g, w) <= 1e-6
     if c % 64 == 0:
         assert torch.equal(got[3].view(torch.int16), K.bf16_split(got[0]).view(torch.int16))
@@ -323,7 +326,7 @@ def test_bn_statistics_of_channels_with_mean_far_from_zero(K, rows, c):
 
 
 @pytest.mark.parametrize("rows,c", [(1000, 64), (777, 3), (4099, 256), (300, 515), (50, 12), (9000, 128), (64, 8)])
-def test_bn_stats_apply_bwd(K, rows, c):
+def test_bn_stats_apply_bwd_against_the_oracle(K, rows, c):
     x = rnd(rows, c) * 2 + 0.5
     gamma, beta = rnd(c, seed=1) * 0.3 + 1, rnd(c, seed=2) * 0.1
     rm, rv = rnd(c, seed=3) * 0.1, rnd(c, seed=4).abs() + 0.5
@@ -345,17 +348,17 @@ def test_bn_stats_apply_bwd(K, rows, c):
     sc2, sh2 = rnd(c, seed=6), rnd(c, seed=7)
     for mode, relu in ((S.RES_NONE, False), (S.RES_TENSOR, True), (S.RES_AFFINE, True)):
         kw = dict(res_mode=mode, res=res, scale2=sc2, shift2=sh2, relu=relu)
-        o = K.bn_apply(c_(x), sc.float().cuda(), sh.float().cuda(), **{k: (v.cuda() if torch.is_tensor(v) else v) for k, v in kw.items()})
-        o_ref = S.bn_apply(d(x), sc, sh, **{k: (v.double() if torch.is_tensor(v) else v) for k, v in kw.items()})
+        o = K.bn_apply(c_(x), sc.float().cuda(), sh.float().cuda(), **{k: (v.cuda() if torch.is_tensor(v) else v) for k, v in kw.items()})[0]
+        o_ref = S.bn_apply(d(x), sc, sh, **{k: (v.double() if torch.is_tensor(v) else v) for k, v in kw.items()})[0]
         assert rel_err(o, o_ref) <= 2e-6
     dout, mask = rnd(rows, c, seed=8), rnd(rows, c, seed=9)
     dres0 = rnd(rows, c, seed=10)
     for use_mask, acc in ((True, False), (False, True)):
         dres_c, dres_d = c_(dres0), d(dres0)
         mk = mask if use_mask else None
-        dy, dg, db = K.bn_bwd(c_(dout), None if mk is None else c_(mk), c_(x), mean.float().cuda(), invstd.float().cuda(), c_(gamma),
-                              dres=dres_c, dres_accumulate=acc)
-        dy_r, dg_r, db_r = S.bn_bwd(d(dout), None if mk is None else d(mk), d(x), mean, invstd, d(gamma), dres=dres_d, dres_accumulate=acc)
+        dy, dg, db, _ = K.bn_bwd(c_(dout), None if mk is None else c_(mk), c_(x), mean.float().cuda(), invstd.float().cuda(), c_(gamma),
+                                 dres=dres_c, dres_accumulate=acc)
+        dy_r, dg_r, db_r, _ = S.bn_bwd(d(dout), None if mk is None else d(mk), d(x), mean, invstd, d(gamma), dres=dres_d, dres_accumulate=acc)
         assert rel_err(dy, dy_r) <= 1e-5 and rel_err(dg, dg_r) <= 1e-5 and rel_err(db, db_r) <= 1e-5
         assert rel_err(dres_c, dres_d) <= 1e-6
 
@@ -376,13 +379,14 @@ def test_bn_rowmap_data_bn_addressing(K):
 
 
 @pytest.mark.parametrize("rows,c", [(1000, 64), (4099, 256), (777, 128), (9001, 16), (50, 12), (333, 515), (37, 32)])
-def test_relu_bit_mask_matches_tensor_mask(K, rows, c):
-    """agcn_bn_apply_mask / agcn_bn_bwd_bits: the ReLU mask as one bit per element gives bit-identical results to the fp32
+def test_relu_bit_mask_from_bn_apply_matches_tensor_mask(K, rows, c):
+    """agcn_bn_apply / agcn_bn_bwd with mask_bits: the ReLU mask as one bit per element gives bit-identical results to the fp32
     tensor mask (rows * c not a multiple of 32 included); unsupported layouts return no bit mask."""
     y, res = (rnd(rows, c) * 2).cuda(), rnd(rows, c, seed=1).cuda()
     sc, sh = (rnd(c, seed=2) * 0.3 + 1).cuda(), (rnd(c, seed=3) * 0.1).cuda()
-    out_ref = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True)
-    out, bits = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
+    out_ref, no_bits, _ = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True)
+    out, bits, _ = K.bn_apply(y, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
+    assert no_bits is None
     assert torch.equal(out, out_ref)
     if c % 4 or 256 % (c // 4):
         assert bits is None
@@ -398,7 +402,8 @@ def test_relu_bit_mask_matches_tensor_mask(K, rows, c):
         dres_a, dres_b = rnd(rows, c, seed=8).cuda(), rnd(rows, c, seed=8).cuda()
         a = K.bn_bwd(dout, out_ref, y, mean, invstd, gamma, dres=dres_a, dres_accumulate=acc)
         b = K.bn_bwd(dout, None, y, mean, invstd, gamma, dres=dres_b, dres_accumulate=acc, mask_bits=bits)
-        for u, v in zip(a, b):
+        assert a[3] is None and b[3] is None
+        for u, v in zip(a[:3], b[:3]):
             assert torch.equal(u, v)
         assert torch.equal(dres_a, dres_b)
 
@@ -458,8 +463,8 @@ def test_tf32_tensor_core_path(K, nb, t_in, v, cin, cout, taps, stride):
 
 
 @pytest.mark.parametrize("groups,rpg,c,res_mode", [(4, 75, 256, 1), (3, 50, 64, 2), (2, 33, 128, 0), (64, 3750, 256, 1)])
-def test_bn_apply_pool_tail_and_its_backward(K, groups, rpg, c, res_mode):
-    """agcn_bn_apply_pool / agcn_bn_bwd_pool (the model's fused tail) against bn_apply + pool_fwd and pool_bwd + bn_bwd."""
+def test_bn_apply_pool_tail_and_pooled_bn_bwd(K, groups, rpg, c, res_mode):
+    """agcn_bn_apply_pool / agcn_bn_bwd with pool_rows (the model's fused tail) against bn_apply + pool_fwd and pool_bwd + bn_bwd."""
     rows = groups * rpg
     assert K.bn_pool_supported(rows, c)
     y, res = rnd(rows, c).cuda(), rnd(rows, c, seed=1).cuda()
@@ -467,7 +472,7 @@ def test_bn_apply_pool_tail_and_its_backward(K, groups, rpg, c, res_mode):
     sc2, sh2 = (rnd(c, seed=4) * 0.3 + 1).cuda(), (rnd(c, seed=5) * 0.2).cuda()
     kw = dict(res_mode=res_mode, res=res if res_mode else None, scale2=sc2 if res_mode == 2 else None, shift2=sh2 if res_mode == 2 else None)
     pooled, bits = K.bn_apply_pool(y, sc, sh, groups=groups, **kw)
-    out, bits_ref = K.bn_apply(y, sc, sh, relu=True, want_mask=True, **kw)
+    out, bits_ref, _ = K.bn_apply(y, sc, sh, relu=True, want_mask=True, **kw)
     assert torch.equal(bits, bits_ref)
     assert rel_err(pooled, out.double().reshape(groups, rpg, c).mean(1)) <= 2e-6
     d_pooled = rnd(groups, c, seed=6).cuda()
@@ -476,7 +481,8 @@ def test_bn_apply_pool_tail_and_its_backward(K, groups, rpg, c, res_mode):
     dres_a, dres_b = torch.empty_like(y), torch.empty_like(y)
     got = K.bn_bwd(d_pooled, None, y, mean, invstd, gamma, dres=dres_a, mask_bits=bits, pool_rows=rpg)
     want = K.bn_bwd(d_full, None, y, mean, invstd, gamma, dres=dres_b, mask_bits=bits)
-    for a, b in zip(got, want):
+    assert got[3] is None and want[3] is None
+    for a, b in zip(got[:3], want[:3]):
         assert rel_err(a, b) <= 2e-6
     assert rel_err(dres_a, dres_b) <= 1e-6
 

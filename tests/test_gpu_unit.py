@@ -312,7 +312,7 @@ class _MirrorSync:
 @pytest.mark.gpu
 @pytest.mark.parametrize("start,shape", [(64, (2, 24, 25, 3)), (16, (1, 20, 20, 3))])
 def test_sync_batchnorm_halves_on_mirrored_ranks(pkg, start, shape):
-    """agcn_bn_stats_partials / agcn_bn_finalize over concatenated partials / agcn_bn_bwd_sync phases 1 and 2 (SURVEY 8e optional SyncBN);
+    """agcn_bn_stats_partials / agcn_bn_finalize over concatenated partials / agcn_bn_bwd phases 1 and 2 (SURVEY 8e optional SyncBN);
     the real two-rank exchange is tested on gloo (tests/test_distributed_cpu.py)."""
     import copy
     from fusion_gcn_b200 import capi, graph as G

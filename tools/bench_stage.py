@@ -119,13 +119,13 @@ def main():
             report(f"bn_apply_res_{tag}", ms, act * 3, 0)
             ms = timeit(lambda: K.bn_bwd(dout, msk, x, mean, invstd, gamma), once)
             report(f"bn_bwd_{tag}", ms, act * 7, 0)              # two passes over (dout, mask, y) + dy
-            _, bits = K.bn_apply(x, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
+            _, bits, _ = K.bn_apply(x, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True)
             ms = timeit(lambda: K.bn_apply(x, sc, sh, res_mode=K.RES_TENSOR, res=res, relu=True, want_mask=True), once)
             report(f"bn_apply_res_mask_{tag}", ms, act * 3, 0)
             ms = timeit(lambda: K.bn_bwd(dout, None, x, mean, invstd, gamma, mask_bits=bits), once)
             report(f"bn_bwd_bits_{tag}", ms, act * 5, 0)         # two passes over (dout, y) + dy (+ 1/32 for the bits)
             if bits is not None:                                 # two BatchNorms over one upstream gradient (agcn_bn_bwd_bits_dual)
-                ms = timeit(lambda: K.bn_bwd_dual(dout, bits, (x, mean, invstd, gamma), (res, mean, invstd, gamma)), once)
+                ms = timeit(lambda: K.bn_bwd_dual(dout, (x, mean, invstd, gamma), (res, mean, invstd, gamma), mask_bits=bits), once)
                 report(f"bn_bwd_dual_{tag}", ms, act * 8, 0)     # two passes over (dout, y_a, y_b) + dy_a + dy_b
             del res, dout, msk
         del x
