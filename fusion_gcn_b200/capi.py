@@ -63,9 +63,11 @@ SIGNATURES = {
     "agcn_bucket_copy": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_float, _c_void_p]),
     "agcn_optim_chunk": (_c_int, []),
     "agcn_optim_sgd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_double, _c_void_p, _c_double, _c_double, _c_double, _c_int, _c_int,
-                                _c_void_p, _c_void_p, _c_void_p]),
+                                _c_int, _c_void_p, _c_void_p, _c_void_p]),
     "agcn_optim_adam": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_double, _c_void_p, _c_double, _c_double, _c_double, _c_double, _c_int,
-                                 _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
+                                 _c_int, _c_int, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
+    "agcn_optim_asgd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_double, _c_void_p, _c_double, _c_double, _c_double, _c_double, _c_int]
+                        + [_c_void_p] * 7),
 }
 
 _lock = threading.Lock()

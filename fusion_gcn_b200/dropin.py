@@ -55,7 +55,7 @@ def install_shims(reference_root: str, host_stubs: bool = True) -> None:
 def install(reference_root: str, precision="fp32", host_stubs: bool = True, fused_optimizers: bool = False, prefetch: bool = False,
             recompute: bool = False) -> dict:
     """Rebinds the reference's unit / backbone classes to the B200 implementations.  Returns the patched modules.
-    ``fused_optimizers``: the YAML optimizer names SGD / ADAM / ADAMW (torch_src/session_helper.py:48-53) build the multi-tensor
+    ``fused_optimizers``: the YAML optimizer names SGD / ADAM / ADAMW / ASGD (torch_src/session_helper.py:48-53) build the multi-tensor
     classes of fusion_gcn_b200.optim.  ``prefetch``: the sessions' ``DataLoader`` (session/training.py:18-25, evaluation.py:20-24,
     debugging.py:15-21) becomes fusion_gcn_b200.pipeline.PrefetchLoader (same batches, pinned staging + asynchronous H2D)."""
     from . import modules, modules_original

@@ -288,26 +288,40 @@ int agcn_linear_ce_fwd(const float* x, const float* w, const float* bias, const 
 int agcn_linear_ce_bwd(const float* x, const float* w, const float* dlogits, const float* grad_loss,
                        float* dw, float* dbias, float* dx, int n, int cin, int ncls, void* stream);
 
-/* ---- multi-tensor optimizer steps (torch_src/session_helper.py:48-82 builds torch.optim.{SGD, Adam, AdamW};
- * torch_src/session/procedures/step.py:48-49,67-71 steps them, under GradScaler with --mixed_precision) ------------
+/* ---- multi-tensor optimizer steps (torch_src/session_helper.py:48-53 is the table of torch.optim.{SGD, Adam, AdamW, ASGD} the
+ * YAML `optimizer` key selects, :56-82 builds it; torch_src/session/procedures/step.py:48-49,67-71 steps it, under GradScaler with
+ * --mixed_precision) ------------
  * ONE launch updates every parameter tensor of a group.  `table`: device array of rows
  *     { float* param; const float* grad; float* state1; float* state2; long long numel; }      (40 bytes each)
- * `items`: device array of (row index, chunk index) int pairs, one per agcn_optim_chunk() elements of every tensor.
+ * except for AMSGrad Adam (below).  `items`: device array of (row index, chunk index) int pairs, one per agcn_optim_chunk()
+ * elements of every tensor.
  * lr_dev (may be NULL) overrides `lr` with a device scalar, so a captured CUDA graph follows a learning-rate schedule.
  * grad_scale / found_inf (may be NULL) are GradScaler's device scalars: gradients are divided by *grad_scale and the
- * whole step is skipped when *found_inf != 0 -- no host synchronisation.  Hyper-parameters are doubles (Python floats): 1 - beta
- * and the Adam bias corrections are formed in double before they are rounded to fp32, as torch.optim does on the host.
+ * whole step is skipped when *found_inf != 0 -- no host synchronisation.  maximize != 0 negates the unscaled gradient before
+ * anything else uses it.  Hyper-parameters are doubles (Python floats): 1 - beta and the Adam bias corrections are formed in
+ * double before they are rounded to fp32, as torch.optim does on the host.
  * SGD  (torch/optim/sgd.py): g += wd*p; buf = first_step ? g : momentum*buf + (1-dampening)*g (state1);
  *                            g = nesterov ? g + momentum*buf : buf; p -= lr*g.
  * Adam (torch/optim/adam.py): state1 = exp_avg, state2 = exp_avg_sq, *step_dev = steps completed before this one (the caller
- *                            increments it afterwards); decoupled != 0 is AdamW (p *= 1 - lr*wd instead of g += wd*p). */
+ *                            increments it afterwards); decoupled != 0 is AdamW (p *= 1 - lr*wd instead of g += wd*p).
+ *                            amsgrad != 0: the rows carry a third state tensor,
+ *     { float* param; const float* grad; float* exp_avg; float* exp_avg_sq; float* max_exp_avg_sq; long long numel; }  (48 bytes)
+ *                            max_exp_avg_sq = max(max_exp_avg_sq, exp_avg_sq) divides the step in place of exp_avg_sq.
+ * ASGD (torch/optim/asgd.py, capturable form): state1 = ax, state2 unused.  eta / mu / step: ONE set of fp32 device scalars for the
+ *                            group (torch keeps one per parameter, all equal).  g += wd*p; p *= 1 - lambd*eta; p -= eta*g;
+ *                            ax += (p - ax)*mu; then, once for the launch, step += 1, eta = lr / (1 + lambd*lr*step)^alpha,
+ *                            mu = 1 / max(1, step - t0).  done: a device int that is zero before the call; the launch leaves it
+ *                            zero (the last block to finish counts itself there and advances the scalars).                      */
 int agcn_optim_chunk(void);
 int agcn_optim_sgd(const void* table, const int* items, int nitems, double lr, const float* lr_dev,
-                   double momentum, double dampening, double weight_decay, int nesterov, int first_step,
+                   double momentum, double dampening, double weight_decay, int nesterov, int first_step, int maximize,
                    const float* grad_scale, const float* found_inf, void* stream);
 int agcn_optim_adam(const void* table, const int* items, int nitems, double lr, const float* lr_dev,
-                    double beta1, double beta2, double eps, double weight_decay, int decoupled,
+                    double beta1, double beta2, double eps, double weight_decay, int decoupled, int amsgrad, int maximize,
                     const float* step_dev, const float* grad_scale, const float* found_inf, void* stream);
+int agcn_optim_asgd(const void* table, const int* items, int nitems, double lr, const float* lr_dev,
+                    double lambd, double alpha, double t0, double weight_decay, int maximize,
+                    float* eta, float* mu, float* step, int* done, const float* grad_scale, const float* found_inf, void* stream);
 
 /* Node mixing with ONE fixed matrix for the whole batch -- STGCNGraphConvolution's support . adj^T
  * (torch_src/models/mmargcn/graph_convolution.py:45) and its input gradient:
