@@ -183,13 +183,13 @@ int agcn_joint_mix_big(const float* in, const float* mats, float* out, int nb, i
     p.alpha = 1.f;
     const long long mat = (long long)v * v;
     if (mode == AGCN_MIX_AGG_FWD) {
-        // out[n][t][v][k*W + c] = sum_u G[n][k][u][v] * in[n][t][u][c]: batch (n*t, k), A(m = v, k = u) = G[u][v]
+        // out[n][t][v][k*W + c] (+)= sum_u G[n][k][u][v] * in[n][t][u][c]: batch (n*t, k), A(m = v, k = u) = G[u][v]
         p.a = mats; p.b = in; p.c = out;
         p.batch2 = 3; p.segs = 1; p.m = v; p.n = width; p.k = v;
         p.a_b1 = 0; p.a_b2 = mat; p.a_m = 1; p.a_k = v;
         p.b_b1 = (long long)v * ldin; p.b_b2 = 0; p.b_k = ldin; p.b_n = 1;
         p.c_b1 = (long long)v * ldout; p.c_b2 = width; p.c_m = ldout;
-        p.accumulate = 0;
+        p.accumulate = accumulate;
         // batch1 runs over (n, t): the matrix stride follows n only -> one launch per sample block of timesteps
         for (int n = 0; n < nb; ++n) {
             BigGemm q = p;
@@ -219,10 +219,11 @@ int agcn_joint_mix_big(const float* in, const float* mats, float* out, int nb, i
         return AGCN_OK;
     }
     // SCORE_BWD: in = [theta_0 phi_0 theta_1 phi_1 theta_2 phi_2], mats = dS
-    //   out[.., u, theta_k c] = sum_v dS[k][u][v] * in[.., v, phi_k c];   out[.., v, phi_k c] = sum_u dS[k][u][v] * in[.., u, theta_k c]
+    //   out[.., u, theta_k c] (+)= sum_v dS[k][u][v] * in[.., v, phi_k c];   out[.., v, phi_k c] (+)= sum_u dS[k][u][v] * in[.., u, theta_k c]
+    // the theta and phi slots are disjoint columns, so each of the two GEMMs adds into its own slot
     for (int n = 0; n < nb; ++n) {
         BigGemm q{};
-        q.alpha = 1.f; q.accumulate = 0;
+        q.alpha = 1.f; q.accumulate = accumulate;
         q.batch2 = 3; q.segs = 1; q.m = v; q.n = width; q.k = v;
         q.b_b1 = (long long)v * ldin; q.b_b2 = 2 * width; q.b_k = ldin; q.b_n = 1;
         q.c_b1 = (long long)v * ldout; q.c_b2 = 2 * width; q.c_m = ldout;

@@ -158,7 +158,8 @@ int agcn_attention_bwd(const float* dg_part, const float* p, float* dg_sum, floa
  * precision: AGCN_PREC_FP32 / AGCN_PREC_TF32 run the mix on the tensor cores (3xTF32 / single-pass TF32) when width is a
  * multiple of 32 (AGCN_MIX_AGG_FWD / AGCN_MIX_AGG_BWD) or of 16 (AGCN_MIX_SCORE_BWD) and the workspace holds
  * agcn_joint_mix_workspace_bytes(nb) bytes (zero-padded copies of the matrices); every other case and
- * AGCN_PREC_FP32_FFMA use the FFMA kernel (workspace may then be NULL).                                                     */
+ * AGCN_PREC_FP32_FFMA use the FFMA kernel (workspace may then be NULL).
+ * accumulate != 0 adds into out instead of overwriting it, in every mode and for every V.                                     */
 size_t agcn_joint_mix_workspace_bytes(int nb);
 int agcn_joint_mix(const float* in, const float* mats, float* out,
                    int nb, int t, int v, int ldin, int ldout, int width, int mode, int accumulate,
