@@ -22,6 +22,17 @@ RES_NONE, RES_TENSOR, RES_AFFINE = 0, 1, 2
 _c_int, _c_ll, _c_float, _c_void_p, _c_size_t = ctypes.c_int, ctypes.c_longlong, ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t
 _c_double = ctypes.c_double
 
+
+class _c_count_ptr:
+    """agcn_bn_bwd's global_rows: a device address (int) or None.  The slot held the row count as a host double before the count moved
+    to the device; a Python number there (a caller written for that form) binds as NULL -- never read in phases 0 and 1, refused by
+    phase 2 -- rather than as an address the kernel would read."""
+
+    @classmethod
+    def from_param(cls, value):
+        return None if isinstance(value, float) else _c_void_p.from_param(value)
+
+
 # name -> (restype, argtypes); mirrors include/agcn_b200.h one to one
 SIGNATURES = {
     "agcn_version": (_c_int, []),
@@ -45,10 +56,11 @@ SIGNATURES = {
     "agcn_bn_workspace_bytes": (_c_size_t, [_c_int]),
     "agcn_bn_stats": (_c_int, [_c_void_p, _c_int, _c_int, _c_ll, _c_int] + [_c_void_p] * 5 + [_c_float, _c_float, _c_int]
                       + [_c_void_p] * 4 + [_c_void_p, _c_size_t, _c_void_p]),
-    "agcn_bn_finalize": (_c_int, [_c_void_p, _c_int, _c_ll, _c_int] + [_c_void_p] * 5 + [_c_float, _c_float] + [_c_void_p] * 5),
+    "agcn_bn_finalize": (_c_int, [_c_void_p, _c_int, _c_ll, _c_int] + [_c_void_p] * 5 + [_c_float, _c_float] + [_c_void_p] * 4
+                         + [_c_int, _c_void_p, _c_void_p]),
     "agcn_bn_apply": (_c_int, [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int] + [_c_void_p] * 3 + [_c_int, _c_int, _c_ll, _c_int, _c_void_p]),
     "agcn_bn_mask_words": (_c_size_t, [_c_int] * 3),
-    "agcn_bn_bwd": (_c_int, [_c_void_p] * 12 + [_c_int, _c_int, _c_int, _c_int, _c_ll, _c_int, _c_int, _c_int, _c_void_p, _c_double,
+    "agcn_bn_bwd": (_c_int, [_c_void_p] * 12 + [_c_int, _c_int, _c_int, _c_int, _c_ll, _c_int, _c_int, _c_int, _c_void_p, _c_count_ptr,
                              _c_void_p, _c_size_t, _c_void_p]),
     "agcn_pool_fwd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p]),
     "agcn_pool_bwd": (_c_int, [_c_void_p, _c_void_p, _c_int, _c_int, _c_int, _c_void_p]),

@@ -238,6 +238,25 @@ __device__ __forceinline__ void reduce_partials4(const float* part, int P, int C
     a_out = a; b_out = b;
 }
 
+// running statistics of channel c from the batch mean / biased variance over `count` rows (unbiased variance, as nn.BatchNorm)
+__device__ __forceinline__ void update_running(int c, double mean, double var, double count, float momentum,
+                                               float* running_mean, float* running_var) {
+    const double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
+    running_mean[c] = (float)((1.0 - momentum) * running_mean[c] + momentum * mean);
+    running_var[c] = (float)((1.0 - momentum) * running_var[c] + momentum * unbiased);
+}
+
+__device__ __forceinline__ void write_affine(int c, double mean, double var, float eps, const float* gamma, const float* beta,
+                                             float* scale, float* shift, float* save_mean, float* save_invstd) {
+    const double invstd = 1.0 / sqrt(var + (double)eps);
+    const float g = gamma ? gamma[c] : 1.f, b = beta ? beta[c] : 0.f;
+    const float sc = (float)(g * invstd);
+    scale[c] = sc;
+    shift[c] = (float)(b - mean * g * invstd);
+    if (save_mean) save_mean[c] = (float)mean;
+    if (save_invstd) save_invstd[c] = (float)invstd;
+}
+
 __global__ void __launch_bounds__(256) bn_finalize_kernel(const float* part, int P, int C, double count,
                                    const float* gamma, const float* beta, float* running_mean, float* running_var,
                                    long long* nbt, float momentum, float eps, int training,
@@ -262,22 +281,40 @@ __global__ void __launch_bounds__(256) bn_finalize_kernel(const float* part, int
             var = q / count - d * d;
         }
         if (var < 0.0) var = 0.0;
-        if (running_mean != nullptr) {
-            const double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-            running_mean[c] = (float)((1.0 - momentum) * running_mean[c] + momentum * mean);
-            running_var[c] = (float)((1.0 - momentum) * running_var[c] + momentum * unbiased);
-        }
+        if (running_mean != nullptr) update_running(c, mean, var, count, momentum, running_mean, running_var);
     } else {
         mean = running_mean[c];
         var = running_var[c];
     }
-    const double invstd = 1.0 / sqrt(var + (double)eps);
-    const float g = gamma ? gamma[c] : 1.f, b = beta ? beta[c] : 0.f;
-    const float sc = (float)(g * invstd);
-    scale[c] = sc;
-    shift[c] = (float)(b - mean * g * invstd);
-    if (save_mean) save_mean[c] = (float)mean;
-    if (save_invstd) save_invstd[c] = (float)invstd;
+    write_affine(c, mean, var, eps, gamma, beta, scale, shift, save_mean, save_invstd);
+}
+
+// Synchronised BatchNorm, agcn_bn_finalize phase 1: the partials of this rank reduced to its raw moments in fp64 -- moments[c] = sum x,
+// moments[C + c] = sum x^2 (reduce_partials4: the partial order and formulas of phase 0), moments[2C] = rows.  These add across ranks.
+__global__ void __launch_bounds__(256) bn_moments_kernel(const float* part, int P, int C, double rows, double* moments) {
+    const int c = blockIdx.x * kFinCh + threadIdx.x % kFinCh;
+    double a, b;
+    reduce_partials4(part, P, C, c, a, b);
+    if (blockIdx.x == 0 && threadIdx.x == 0) moments[2 * C] = rows;
+    if (c >= C || threadIdx.x >= kFinCh) return;
+    moments[c] = a;
+    moments[C + c] = b;
+}
+
+// phase 2: the statistics from the moments summed over all ranks (their row count included), as phase 0 forms them from its own sums
+__global__ void __launch_bounds__(256) bn_finalize_moments_kernel(const double* moments, int C, const float* gamma, const float* beta,
+                                                                  float* running_mean, float* running_var, long long* nbt,
+                                                                  float momentum, float eps,
+                                                                  float* scale, float* shift, float* save_mean, float* save_invstd) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c == 0 && nbt != nullptr) *nbt += 1;
+    if (c >= C) return;
+    const double count = moments[2 * C];
+    const double mean = moments[c] / count;
+    double var = moments[C + c] / count - mean * mean;
+    if (var < 0.0) var = 0.0;
+    if (running_mean != nullptr) update_running(c, mean, var, count, momentum, running_mean, running_var);
+    write_affine(c, mean, var, eps, gamma, beta, scale, shift, save_mean, save_invstd);
 }
 
 // bf16 pieces of four fp32 values, as the parity modes' converters form them (tc_common.cuh bf16_split8): h = bf16(x), m = bf16(x - h),
@@ -419,12 +456,16 @@ __global__ void pool_finalize_kernel(const float* part, float* pooled, int P, in
 
 // coef[0][c] = gamma*invstd, coef[1][c] = s1/m, coef[2][c] = s2/m * invstd, coef[3][c] = mean;  dgamma = s2, dbeta = s1.
 // frozen: mean / invstd are constants (eval-mode BatchNorm on its running statistics), so dy = gamma*invstd*g: coef[1] = coef[2] = 0.
+// DEV_COUNT (agcn_bn_bwd phase 2): the row count is read from the device (*count_dev, the all-reduced count of the forward's moments).
+template <bool DEV_COUNT>
 __global__ void __launch_bounds__(256) bn_bwd_finalize_kernel(const float* part, int P, int C, double count, const float* gamma,
-                                       const float* mean, const float* invstd, float* dgamma, float* dbeta, float* coef, int frozen) {
+                                       const float* mean, const float* invstd, float* dgamma, float* dbeta, float* coef, int frozen,
+                                       const double* count_dev = nullptr) {
     const int c = blockIdx.x * kFinCh + threadIdx.x % kFinCh;
     double s1, s2;
     reduce_partials(part, P, C, c, s1, s2);
     if (c >= C || threadIdx.x >= kFinCh) return;
+    if (DEV_COUNT) count = *count_dev;
     if (dbeta) dbeta[c] = (float)s1;
     if (dgamma) dgamma[c] = (float)s2;
     const float is = invstd[c];
@@ -705,11 +746,28 @@ extern "C" AGCN_API int agcn_bn_stats(const float* x, int outer, int inner, long
 extern "C" AGCN_API int agcn_bn_finalize(const float* part, int nparts, long long rows, int channels,
                                 const float* gamma, const float* beta, float* running_mean, float* running_var,
                                 long long* num_batches_tracked, float momentum, float eps,
-                                float* scale, float* shift, float* save_mean, float* save_invstd, void* stream) {
-    AGCN_REQUIRE(part && scale && shift, AGCN_ERR_NULL, "agcn_bn_finalize: null pointer");
-    AGCN_REQUIRE(nparts > 0 && rows > 0 && channels > 0, AGCN_ERR_BAD_SHAPE, "agcn_bn_finalize: bad shape nparts=%d rows=%lld channels=%d",
+                                float* scale, float* shift, float* save_mean, float* save_invstd,
+                                int phase, double* moments, void* stream) {
+    AGCN_REQUIRE(phase >= 0 && phase <= 2, AGCN_ERR_UNSUPPORTED, "agcn_bn_finalize: phase %d", phase);
+    AGCN_REQUIRE(phase == 0 || moments, AGCN_ERR_NULL, "agcn_bn_finalize: phase %d needs moments", phase);
+    AGCN_REQUIRE(phase == 0 || (reinterpret_cast<uintptr_t>(moments) & 7u) == 0, AGCN_ERR_MISALIGNED,
+                 "agcn_bn_finalize: moments must be 8-byte aligned");
+    AGCN_REQUIRE(phase == 1 || (scale && shift), AGCN_ERR_NULL, "agcn_bn_finalize: null pointer");
+    AGCN_REQUIRE(channels > 0, AGCN_ERR_BAD_SHAPE, "agcn_bn_finalize: bad shape channels=%d", channels);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (phase == 2) {          // part / nparts / rows are not read: the count comes with the moments
+        bn_finalize_moments_kernel<<<ceil_div(channels, 256), 256, 0, s>>>(moments, channels, gamma, beta, running_mean, running_var,
+                                                                           num_batches_tracked, momentum, eps, scale, shift, save_mean, save_invstd);
+        return check_launch("agcn_bn_finalize(phase 2)");
+    }
+    AGCN_REQUIRE(part, AGCN_ERR_NULL, "agcn_bn_finalize: null pointer");
+    AGCN_REQUIRE(nparts > 0 && rows > 0, AGCN_ERR_BAD_SHAPE, "agcn_bn_finalize: bad shape nparts=%d rows=%lld channels=%d",
                  nparts, rows, channels);
-    bn_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, static_cast<cudaStream_t>(stream)>>>(
+    if (phase == 1) {
+        bn_moments_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part, nparts, channels, (double)rows, moments);
+        return check_launch("agcn_bn_finalize(phase 1)");
+    }
+    bn_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(
         part, nparts, channels, (double)rows, gamma, beta, running_mean, running_var, num_batches_tracked, momentum, eps, 1,
         scale, shift, save_mean, save_invstd, nullptr, 1);
     return check_launch("agcn_bn_finalize");
@@ -756,13 +814,14 @@ extern "C" AGCN_API int agcn_bn_apply(const float* y, const float* scale, const 
 
 // phase 0: the whole backward.  Synchronised BatchNorm (statistics over all ranks) splits it around the caller's all-reduce:
 // phase 1 = column sums only (dbeta = sum g, dgamma = sum g xhat of THIS rank's rows), phase 2 = the apply pass from
-// global_sums [2][C] = (sum g | sum g xhat) over all ranks and the global row count.
+// global_sums [2][C] = (sum g | sum g xhat) over all ranks and the global row count, read on the device (global_rows: the count slot of
+// the forward's all-reduced moments), so that nothing comes back to the host and the step stays capturable.
 // pool_rows > 0: dout is the gradient of the fused mean pool, [inner / pool_rows][C], broadcast over the rows of each group.
 extern "C" AGCN_API int agcn_bn_bwd(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
                                     const float* save_mean, const float* save_invstd, const float* gamma,
                                     float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
                                     int frozen_stats, int outer, int inner, long long outer_stride, int channels, int pool_rows,
-                                    int phase, const float* global_sums, double global_rows,
+                                    int phase, const float* global_sums, const double* global_rows,
                                     void* workspace, size_t workspace_bytes, void* stream) {
     int rc = check_map("agcn_bn_bwd", outer, inner, outer_stride, channels);
     if (rc) return rc;
@@ -772,6 +831,10 @@ extern "C" AGCN_API int agcn_bn_bwd(const float* dout, const float* mask_out, co
     AGCN_REQUIRE(!(mask_out && mask_bits), AGCN_ERR_UNSUPPORTED, "agcn_bn_bwd: mask_out and mask_bits are alternatives, not both");
     AGCN_REQUIRE(phase != 1 || (dgamma && dbeta), AGCN_ERR_NULL, "agcn_bn_bwd: phase 1 writes dgamma / dbeta");
     AGCN_REQUIRE(!dy_split || dy, AGCN_ERR_NULL, "agcn_bn_bwd: dy_split needs dy");
+    AGCN_REQUIRE(phase != 2 || (global_sums && global_rows), AGCN_ERR_NULL,
+                 "agcn_bn_bwd: phase 2 needs the all-reduced sums and the global row count");
+    AGCN_REQUIRE(phase != 2 || (reinterpret_cast<uintptr_t>(global_rows) & 7u) == 0, AGCN_ERR_MISALIGNED,
+                 "agcn_bn_bwd: global_rows must be 8-byte aligned");
     AGCN_REQUIRE(pool_rows >= 0 && (pool_rows == 0 || (outer == 1 && inner % pool_rows == 0)), AGCN_ERR_BAD_SHAPE, "agcn_bn_bwd: bad pooled shape");
     AGCN_REQUIRE(pool_rows == 0 || mask_bits, AGCN_ERR_NULL, "agcn_bn_bwd: a pooled gradient needs mask_bits");
     AGCN_REQUIRE(dout && y && save_mean && save_invstd && workspace, AGCN_ERR_NULL, "agcn_bn_bwd: null pointer");
@@ -788,13 +851,12 @@ extern "C" AGCN_API int agcn_bn_bwd(const float* dout, const float* mask_out, co
                      "agcn_bn_bwd: mask_bits: layout not supported (agcn_bn_mask_words returned 0)");
     const float bcast_scale = pool_rows > 0 ? 1.f / (float)pool_rows : 1.f;
     if (phase == 2) {
-        AGCN_REQUIRE(global_sums && global_rows >= (double)rows, AGCN_ERR_NULL, "agcn_bn_bwd: phase 2 needs the all-reduced sums and the global row count");
-        bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(global_sums, 1, channels, global_rows, gamma, save_mean, save_invstd,
-                                                                                         nullptr, nullptr, coef, frozen_stats);
+        bn_bwd_finalize_kernel<true><<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(global_sums, 1, channels, 0.0, gamma, save_mean,
+                                                                                               save_invstd, nullptr, nullptr, coef, frozen_stats, global_rows);
     } else {
         rc = launch_colsum<1>(y, dout, mask_out, save_mean, save_invstd, m, rows, part, P, s, mask_bits, pool_rows, bcast_scale);
         if (rc) return rc;
-        bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part, P, channels, (double)rows, gamma, save_mean, save_invstd, dgamma, dbeta, coef, frozen_stats);
+        bn_bwd_finalize_kernel<false><<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part, P, channels, (double)rows, gamma, save_mean, save_invstd, dgamma, dbeta, coef, frozen_stats);
     }
     rc = check_launch("agcn_bn_bwd(finalize)");
     if (rc) return rc;
@@ -840,8 +902,8 @@ extern "C" AGCN_API int agcn_bn_bwd_bits_dual(const float* dout, const unsigned*
     colsum_dual_kernel<<<P, 256, smem, s>>>(y_a, y_b, dout, mask_bits, mean_a, invstd_a, mean_b, invstd_b, channels, rows, part_a, part_b);
     int rc = check_launch("agcn_bn_bwd_bits_dual(sums)");
     if (rc) return rc;
-    bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part_a, P, channels, (double)rows, gamma_a, mean_a, invstd_a, dgamma_a, dbeta_a, coef_a, frozen_stats);
-    bn_bwd_finalize_kernel<<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part_b, P, channels, (double)rows, gamma_b, mean_b, invstd_b, dgamma_b, dbeta_b, coef_b, frozen_stats);
+    bn_bwd_finalize_kernel<false><<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part_a, P, channels, (double)rows, gamma_a, mean_a, invstd_a, dgamma_a, dbeta_a, coef_a, frozen_stats);
+    bn_bwd_finalize_kernel<false><<<ceil_div(channels, kFinCh), kFinCh * kFinLanes, 0, s>>>(part_b, P, channels, (double)rows, gamma_b, mean_b, invstd_b, dgamma_b, dbeta_b, coef_b, frozen_stats);
     rc = check_launch("agcn_bn_bwd_bits_dual(finalize)");
     if (rc) return rc;
     bn_bwd_apply_dual_kernel<<<elementwise_blocks(rows * cq), 256, 0, s>>>(dout, mask_bits, y_a, y_b, coef_a, coef_b, dy_a, dy_b,
@@ -853,7 +915,7 @@ extern "C" AGCN_API int agcn_bn_bwd_bits_dual(const float* dout, const unsigned*
 // The collectives stay with the caller (torch.distributed / NCCL); the library provides the two halves either side of them.
 
 // part4 [P][4][C]: per row-partition p the shifted sum | shifted sum of squares | pivot | row count -- the layout agcn_bn_finalize merges
-// (the same one the convolution epilogue writes), so the partials of several ranks can simply be concatenated.
+// (the same one the convolution epilogue writes), so one finalize (phase 1: this rank's moments) serves both sources.
 __global__ void expand_partials_kernel(const float* part2, const float* x_first_row, int P, int C, long long rows, float* part4) {
     const long long per = (rows + P - 1) / P;
     for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < P * C; idx += gridDim.x * blockDim.x) {

@@ -19,32 +19,42 @@ from . import capi
 
 
 def shard_batch(n_global: int, rank: int, world: int):
-    """Rank r takes samples [r*N/R, (r+1)*N/R) (SURVEY 8e)."""
+    """Rank r takes samples [r*N/R, (r+1)*N/R) (SURVEY 8e).  Equal shards only; see split_batch for any N >= R."""
     if n_global % world:
         raise ValueError(f"global batch {n_global} is not divisible by world size {world}")
     per = n_global // world
     return rank * per, (rank + 1) * per
 
 
+def split_batch(n_global: int, rank: int, world: int):
+    """Rank r's shard of a global batch of N sequences over R ranks, for any N >= R: -> (lo, hi, loss_weight).
+
+    The shards follow ``torch.tensor_split``: the first N mod R ranks take one sequence more.  ``loss_weight`` = n_r * R / N (exactly
+    1.0 for equal shards) is the factor a MEAN-reduced loss of the shard must be multiplied by before ``backward()``: the gradient
+    all-reduce then averages to the gradient of the unsharded batch's mean loss.  Scaling at the all-reduce instead is not enough with
+    synchronised BatchNorm, whose backward adds the ranks' upstream gradients, so every rank's must be on the same scale.
+    ``(loss * loss_weight).backward()`` reaches the fused classifier (``Model.loss``) through its device-side loss gradient."""
+    if not 0 <= rank < world:
+        raise ValueError(f"rank {rank} outside a world of {world}")
+    if n_global < world:
+        raise ValueError(f"global batch {n_global} is smaller than world size {world}: a rank would get no sequence")
+    per, extra = divmod(n_global, world)
+    lo = rank * per + min(rank, extra)
+    hi = lo + per + (1 if rank < extra else 0)
+    return lo, hi, (hi - lo) * world / n_global
+
+
 class SyncBatchNorm:
     """The collectives of a synchronised BatchNorm (``modules.set_sync_batchnorm``): training-mode statistics and their backward sums
-    over all ranks of ``group``, so that a batch sharded over R GPUs normalises exactly like the unsharded batch (SURVEY 8e).  The
-    kernels produce MERGEABLE partials (shifted sums with their pivots and row counts, the layout the convolution epilogue writes
-    anyway), so the forward needs one all-gather of a few KB per BatchNorm and no second pass; the backward all-reduces the two
-    column sums between its sum pass and its apply pass.  Stream-ordered on NCCL: capturable in the step's CUDA graph."""
+    over all ranks of ``group``, so that a batch sharded over R GPUs normalises exactly like the unsharded batch (SURVEY 8e), whether
+    or not the shards are of equal size.  In the forward each rank reduces its partials to fp64 moments (sum x | sum x^2 | rows,
+    2C + 1 doubles: at most 4 KB at C = 256) and all-reduces them; the count travels with the moments to the backward, which
+    all-reduces its two fp32 column sums between its sum pass and its apply pass.  Both payloads have a fixed size whatever the
+    shard or world size.  Stream-ordered on NCCL: capturable in the step's CUDA graph."""
 
     def __init__(self, group=None):
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-
-    def gather_partials(self, part: torch.Tensor) -> torch.Tensor:
-        """[nparts, 4, c] of this rank -> [world * nparts, 4, c] of all ranks (every rank runs the same shapes)."""
-        if self.world == 1:
-            return part
-        part = part.contiguous()
-        out = part.new_empty((self.world * part.shape[0],) + tuple(part.shape[1:]))
-        dist.all_gather_into_tensor(out, part, group=self.group)       # concatenation along dim 0, rank order
-        return out
 
     def all_reduce(self, t: torch.Tensor) -> torch.Tensor:
         if self.world > 1:

@@ -53,21 +53,58 @@ class UnitSpec:
     recompute: bool = False         # do not keep theta / phi (e) and the aggregated tensor (z) for the backward; run their kernels again there
 
 
+class _ShardSync:
+    """The synchronisation of ONE BatchNorm's backward: the group's ``all_reduce`` and that BatchNorm's global row count, taken from
+    the count slot of its forward's all-reduced moments.  ``global_rows`` (CUDA tensors): the device scalar agcn_bn_bwd phase 2 reads,
+    so the count never passes through the host.  ``world`` = global rows / this rank's rows (the world size when the shards are equal):
+    the factor by which a composition on CPU tensors, which counts rows as local rows x ``world``, gets the global count."""
+
+    def __init__(self, sync, count, local_rows):
+        self.all_reduce = sync.all_reduce
+        self.global_rows = count if count.is_cuda else None
+        self.world = sync.world if count.is_cuda else float(count) / local_rows
+
+
+def _sync_finalize(part, rows, gamma, beta, buf: BnBuffers, tracked, sync):
+    """Synchronised BatchNorm statistics: this rank's partials reduced to fp64 moments (sum x | sum x^2 | rows), summed over the ranks
+    with one fixed-size all-reduce whatever the shard sizes, and finalised (agcn_bn_finalize phases 1 and 2).  -> scale, shift,
+    save_mean, save_invstd, and the _ShardSync of this BatchNorm's backward.
+    CPU tensors (gloo groups running the host composition on a CPU stage backend, which has no phase calls): the same moments with the
+    formulas of the phase-1 kernel, finalised as the single partial (sum x, sum x^2, pivot 0, rows) -- the same statistics."""
+    if part.is_cuda:
+        moments = sync.all_reduce(K.bn_moments(part, rows))
+        out = K.bn_finalize_moments(moments, gamma, beta, buf.running_mean, buf.running_var, tracked, BN_MOMENTUM, BN_EPS)
+    else:
+        moments = sync.all_reduce(host_moments(part, rows))
+        c = part.shape[-1]
+        one = torch.stack([moments[:c], moments[c:2 * c], torch.zeros_like(moments[:c]), moments[2 * c:].expand(c)]).unsqueeze(0)
+        out = K.bn_finalize(one, float(moments[2 * c]), gamma, beta, buf.running_mean, buf.running_var, tracked, BN_MOMENTUM, BN_EPS)
+    return tuple(out) + (_ShardSync(sync, moments[2 * part.shape[-1]:], rows),)
+
+
+def host_moments(part, rows):
+    """fp64 moments [2c + 1] = sum x | sum x^2 | rows of CPU partials [nparts, 4, c] (shifted sum | shifted sum of squares | pivot | row
+    count), with the formulas of agcn_bn_finalize phase 1: a = sum_p (n_p piv_p + s1_p), b = sum_p (s2_p + piv_p (2 s1_p + n_p piv_p))."""
+    p = part.double()
+    s1, s2, piv, n = p[:, 0], p[:, 1], p[:, 2], p[:, 3]
+    return torch.cat([(n * piv + s1).sum(0), (s2 + piv * (2 * s1 + n * piv)).sum(0), p.new_full((1,), float(rows))])
+
+
 def _bn_forward(y, gamma, beta, buf: BnBuffers, training: bool, sync=None, rowmap=None, nbt=True):
-    """-> scale, shift, save_mean, save_invstd.  ``sync`` (training mode): the statistics are taken over the rows of ALL ranks -- every
-    rank's mergeable partials are all-gathered and finalised with the global row count (synchronised BatchNorm)."""
+    """-> scale, shift, save_mean, save_invstd, the sync object of this BatchNorm's backward | None.  ``sync`` (training mode): the
+    statistics are taken over the rows of ALL ranks (synchronised BatchNorm, see _sync_finalize); otherwise the last item is None."""
     tracked = buf.num_batches_tracked if nbt else None
     if training and sync is not None:
         part = K.bn_stats_partials(y, rowmap=rowmap)
         rows = (rowmap[0] * rowmap[1]) if rowmap is not None else y.numel() // y.shape[-1]
-        return K.bn_finalize(sync.gather_partials(part), rows * sync.world, gamma, beta, buf.running_mean, buf.running_var, tracked,
-                             BN_MOMENTUM, BN_EPS)
+        return _sync_finalize(part, rows, gamma, beta, buf, tracked, sync)
     return K.bn_stats(y, gamma, beta, buf.running_mean, buf.running_var, tracked, BN_MOMENTUM, BN_EPS, training,
-                      **({} if rowmap is None else dict(rowmap=rowmap)))
+                      **({} if rowmap is None else dict(rowmap=rowmap))) + (None,)
 
 
 def _conv_bn(x, w, bias, gamma, beta, buf: BnBuffers, training: bool, prec: int, sync=None, **kw):
-    """Conv2d -> BatchNorm2d pair (agcn.py:41-51,73-83): y = conv(x) and the BN scale / shift / saved statistics of y.
+    """Conv2d -> BatchNorm2d pair (agcn.py:41-51,73-83): y = conv(x) and the BN scale / shift / saved statistics of y and the sync
+    object of its backward (see _bn_forward).
     In training mode the column sums come out of the convolution's epilogue (conv_fwd_stats) when the kernel covers the
     shape, which saves the separate statistics pass over y."""
     if training:
@@ -75,9 +112,9 @@ def _conv_bn(x, w, bias, gamma, beta, buf: BnBuffers, training: bool, prec: int,
         if part is not None:
             rows = y.numel() // y.shape[-1]
             if sync is not None:
-                part, rows = sync.gather_partials(part), rows * sync.world
+                return y, _sync_finalize(part, rows, gamma, beta, buf, buf.num_batches_tracked, sync)
             return y, K.bn_finalize(part, rows, gamma, beta, buf.running_mean, buf.running_var, buf.num_batches_tracked,
-                                    BN_MOMENTUM, BN_EPS)
+                                    BN_MOMENTUM, BN_EPS) + (None,)
     else:
         y = K.conv_fwd(x, w, bias, precision=prec, **kw)
     return y, _bn_forward(y, gamma, beta, buf, training, sync)
@@ -178,12 +215,12 @@ def gcn_forward(x, adj_a, adj_b, wa, ba, wb, bb, wd, bd, bn_w, bn_b, down_w, dow
         if spec.attention_out is not None:
             spec.attention_out[:] = [p[:, k] for k in range(3)]
         return o
-    y, (sc, sh, mean, invstd) = _conv_bn(z, wdc, bdc, bn_w, bn_b, spec.bn_gcn, spec.training, prec, sync=spec.sync)
+    y, (sc, sh, mean, invstd, bn_sync) = _conv_bn(z, wdc, bdc, bn_w, bn_b, spec.bn_gcn, spec.training, prec, sync=spec.sync)
     # the temporal convolution that follows takes its weight gradient from bf16 pieces of `o` written here, by the pass that
     # produces `o` anyway (agcn_conv_wgrad_presplit): no conversion pass in the weight-gradient kernel
     want_split = want_mask and spec.training and cout % 64 == 0 and prec != K.PREC_FP32_FFMA and prec != K.PREC_TF32
     if spec.has_down:
-        yd, (sc2, sh2, mean2, invstd2) = _conv_bn(x, down_w.reshape(cout, 1, cin), down_b, dbn_w, dbn_b, spec.bn_down, spec.training, prec, sync=spec.sync)
+        yd, (sc2, sh2, mean2, invstd2, _) = _conv_bn(x, down_w.reshape(cout, 1, cin), down_b, dbn_w, dbn_b, spec.bn_down, spec.training, prec, sync=spec.sync)
         o, o_bits, o_split = K.bn_apply(y, sc, sh, want_mask=want_mask, want_split=want_split, res_mode=K.RES_AFFINE, res=yd, scale2=sc2,
                                         shift2=sh2, relu=True)
     else:
@@ -196,7 +233,7 @@ def gcn_forward(x, adj_a, adj_b, wa, ba, wb, bb, wd, bd, bn_w, bn_b, down_w, dow
         # ONE deterministic kernel away from x (and g) -- the backward runs those two kernels again and gets the same bits
         keep = not spec.recompute
         ctx.update(x=x, e=e if keep else None, p=p, g=g, z=z if keep else None, y=y, yd=yd, o=o.detach(), o_bits=o_bits, o_split=o_split,
-                   mean=mean, invstd=invstd, mean2=mean2, invstd2=invstd2, wab=wab, bab=bab, wdc=wdc, nchunk=nchunk, scale=scale, ci=ci)
+                   mean=mean, invstd=invstd, mean2=mean2, invstd2=invstd2, bn_sync=bn_sync, wab=wab, bab=bab, wdc=wdc, nchunk=nchunk, scale=scale, ci=ci)
     return o
 
 
@@ -218,7 +255,7 @@ def gcn_backward(d_o, ctx, bn_w, dbn_w, down_w, spec: UnitSpec, dx=None, need_dx
     if spec.has_down:
         # bn and down.1 both feed the ReLU of agcn.py:113-115: one pair of passes over the shared masked gradient for both backwards
         dy, dgam, dbet, _, dyd, dgam2, dbet2 = K.bn_bwd_dual(d_o, (y, ctx["mean"], ctx["invstd"], bn_w), (ctx["yd"], ctx["mean2"], ctx["invstd2"], dbn_w),
-                                                             mask_out=o, mask_bits=ctx["o_bits"], frozen=frozen, sync=spec.sync)
+                                                             mask_out=o, mask_bits=ctx["o_bits"], frozen=frozen, sync=ctx["bn_sync"])
         wdown = down_w.reshape(cout, 1, cin)
         d_down_w, d_down_b = leaves.run(lambda: K.conv_wgrad(dyd, x, want_bias=frozen, precision=prec), dyd, x)
         if not frozen:
@@ -230,7 +267,7 @@ def gcn_backward(d_o, ctx, bn_w, dbn_w, down_w, spec: UnitSpec, dx=None, need_dx
         if need_dx and dx is None:
             dx = torch.empty_like(x)
         dy, dgam, dbet, _ = K.bn_bwd(d_o, o, y, ctx["mean"], ctx["invstd"], bn_w, dres=dx if need_dx else None, dres_accumulate=have,
-                                     mask_bits=ctx["o_bits"], frozen=frozen, sync=spec.sync)
+                                     mask_bits=ctx["o_bits"], frozen=frozen, sync=ctx["bn_sync"])
         have = have or need_dx
         dgam2 = dbet2 = d_down_w = d_down_b = None
     dz = K.conv_fwd(dy, _t(ctx["wdc"]), precision=prec)                                # [nb,t,v,3*cin]
@@ -294,7 +331,7 @@ def tcn_forward(o, x_res, wt, bt, bn_w, bn_b, wr, br, rbn_w, rbn_b, spec: UnitSp
             res = None
         out = K.conv_fwd_post(o, wtp, bt, scale=sc, shift=sh, res=res, relu=spec.relu_out, t_out=t_out, stride=s, pad=pad, precision=prec)
         return out
-    u, (sc, sh, mean, invstd) = _conv_bn(o, wtp, bt, bn_w, bn_b, spec.bn_tcn, spec.training, prec, sync=spec.sync, t_out=t_out, stride=s, pad=pad)
+    u, (sc, sh, mean, invstd, bn_sync) = _conv_bn(o, wtp, bt, bn_w, bn_b, spec.bn_tcn, spec.training, prec, sync=spec.sync, t_out=t_out, stride=s, pad=pad)
     ur = mean2 = invstd2 = wrp = None
     want_mask = ctx is not None and spec.relu_out
     # the model's tail (agcn.py:194-196): the last unit's output only feeds the global mean pool, so the pooled means and the ReLU
@@ -307,13 +344,13 @@ def tcn_forward(o, x_res, wt, bt, bn_w, bn_b, wr, br, rbn_w, rbn_b, spec: UnitSp
         out, out_bits = apply(u, sc, sh, res_mode=K.RES_TENSOR, res=x_res, relu=spec.relu_out)
     elif spec.residual == "conv":
         wrp = _pack_taps(wr)
-        ur, (sc2, sh2, mean2, invstd2) = _conv_bn(x_res, wrp, br, rbn_w, rbn_b, spec.bn_res, spec.training, prec, sync=spec.sync, t_out=t_out, stride=s, pad=0)
+        ur, (sc2, sh2, mean2, invstd2, _) = _conv_bn(x_res, wrp, br, rbn_w, rbn_b, spec.bn_res, spec.training, prec, sync=spec.sync, t_out=t_out, stride=s, pad=0)
         out, out_bits = apply(u, sc, sh, res_mode=K.RES_AFFINE, res=ur, scale2=sc2, shift2=sh2, relu=spec.relu_out)
     else:
         out, out_bits = apply(u, sc, sh, relu=spec.relu_out)
     if ctx is not None:
         ctx.update(t_o=o.detach(), t_o_shape=tuple(o.shape), t_x=x_res, u=u, ur=ur, out=None if (pool or out_bits is not None or not spec.relu_out) else out.data, out_bits=out_bits, t_mean=mean, t_invstd=invstd,
-                   t_mean2=mean2, t_invstd2=invstd2, wtp=wtp, wrp=wrp, pad=pad, pool_rows=(u.numel() // u.shape[-1] // pool) if pool else 0)
+                   t_mean2=mean2, t_invstd2=invstd2, t_sync=bn_sync, wtp=wtp, wrp=wrp, pad=pad, pool_rows=(u.numel() // u.shape[-1] // pool) if pool else 0)
     return out
 
 
@@ -335,7 +372,7 @@ def tcn_backward(d_out, ctx, bn_w, rbn_w, spec: UnitSpec, need_dres=True, need_d
     # bf16 pieces from the BatchNorm backward below (bit-mask forms only)
     o_split = ctx.get("o_split") if (not frozen and bits is not None) else None
     # pool_rows > 0: d_out is the pooled gradient [groups, c]
-    kw = dict(mask_bits=bits, pool_rows=ctx.get("pool_rows", 0), frozen=frozen, sync=spec.sync, want_split=o_split is not None)
+    kw = dict(mask_bits=bits, pool_rows=ctx.get("pool_rows", 0), frozen=frozen, sync=ctx["t_sync"], want_split=o_split is not None)
     if spec.residual == "identity":
         d_xres = torch.empty_like(x_res) if need_dres else None
         du, dgam, dbet, du_split = K.bn_bwd(d_out, mask, u, ctx["t_mean"], ctx["t_invstd"], bn_w, dres=d_xres, dres_accumulate=False, **kw)
@@ -514,11 +551,11 @@ class DataBnFn(torch.autograd.Function):
             sl = slice(mi * vc, (mi + 1) * vc)
             rowmap = (n, t, m * t * vc, vc)
             xv = x[:, mi]
-            sc, sh, mean, invstd = _bn_forward(xv, gamma[sl], beta[sl], BnBuffers(buf.running_mean[sl], buf.running_var[sl], buf.num_batches_tracked),
+            sc, sh, mean, invstd, bn_sync = _bn_forward(xv, gamma[sl], beta[sl], BnBuffers(buf.running_mean[sl], buf.running_var[sl], buf.num_batches_tracked),
                                                training, sync, rowmap=rowmap, nbt=(mi == 0))
             K.bn_apply(xv, sc, sh, rowmap=rowmap, out=out[:, mi])
-            saved.append((mean, invstd))
-        ctx.x, ctx.gamma, ctx.saved, ctx.training, ctx.sync = x, gamma, saved, training, sync
+            saved.append((mean, invstd, bn_sync))
+        ctx.x, ctx.gamma, ctx.saved, ctx.training = x, gamma, saved, training
         return out.view(n * m, t, v, c)
 
     @staticmethod
@@ -534,9 +571,9 @@ class DataBnFn(torch.autograd.Function):
         for mi in range(m):
             sl = slice(mi * vc, (mi + 1) * vc)
             rowmap = (n, t, m * t * vc, vc)
-            mean, invstd = ctx.saved[mi]
+            mean, invstd, bn_sync = ctx.saved[mi]
             _, dg, db, _ = K.bn_bwd(d_out[:, mi], None, x[:, mi], mean, invstd, gamma[sl], want_dy=need_dx,
-                                    dy=dx[:, mi] if need_dx else None, rowmap=rowmap, frozen=not ctx.training, sync=ctx.sync)
+                                    dy=dx[:, mi] if need_dx else None, rowmap=rowmap, frozen=not ctx.training, sync=bn_sync)
             dgamma[sl] = dg
             dbeta[sl] = db
         return dx, dgamma, dbeta, None, None, None

@@ -70,7 +70,8 @@ def set_sync_batchnorm(module: nn.Module, sync=True) -> nn.Module:
     """Synchronised BatchNorm for every unit (and the model's data_bn) under ``module``: training-mode statistics and their backward
     sums are taken over all ranks of a process group, so a batch sharded over R GPUs normalises exactly like the unsharded batch
     (the reference is single-process: its nn.BatchNorm sees the whole batch, agcn.py:44,78,83,150).  ``sync``: True (default group),
-    a ``distributed.SyncBatchNorm``, or None / False to go back to per-replica statistics.  Every rank must run the same local batch size."""
+    a ``distributed.SyncBatchNorm``, or None / False to go back to per-replica statistics.  The ranks' local batch sizes may differ
+    (``distributed.split_batch``; multiply a mean-reduced loss by its ``loss_weight`` before ``backward()``)."""
     if sync is True:
         from .distributed import SyncBatchNorm
         sync = SyncBatchNorm()

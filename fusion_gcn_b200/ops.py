@@ -218,7 +218,36 @@ def bn_finalize(part, rows, gamma, beta, running_mean, running_var, nbt, momentu
         raise RuntimeError("num_batches_tracked must be int64")
     _call("agcn_bn_finalize", _ptr(part), nparts, int(rows), c, _ptr(gamma), _ptr(beta), _ptr(running_mean), _ptr(running_var),
           _ptr(nbt), float(momentum), float(eps), scale[0].data_ptr(), scale[1].data_ptr(), scale[2].data_ptr(), scale[3].data_ptr(),
-          _stream(), sig=(nparts, c), work=(0.0, 0.0))
+          0, None, _stream(), sig=(nparts, c), work=(0.0, 0.0))
+    return scale[0], scale[1], scale[2], scale[3]
+
+
+def bn_moments(part, rows):
+    """Phase 1 of a synchronised BatchNorm's statistics: the partials of this rank (conv_fwd_stats / bn_stats_partials) reduced to
+    fp64 moments [2c + 1] = sum x per channel | sum x^2 per channel | rows.  The moments of all ranks add up (all-reduce, sum);
+    bn_finalize_moments turns the total into the BatchNorm parameters."""
+    nparts, _, c = part.shape
+    _check(part)
+    moments = torch.empty((2 * c + 1,), device=part.device, dtype=torch.float64)
+    _call("agcn_bn_finalize", _ptr(part), nparts, int(rows), c, None, None, None, None, None, 0.0, 0.0, None, None, None, None,
+          1, moments.data_ptr(), _stream(), sig=(nparts, c, 1), work=(0.0, 0.0))
+    return moments
+
+
+def bn_finalize_moments(moments, gamma, beta, running_mean, running_var, nbt, momentum, eps):
+    """Phase 2: scale, shift, save_mean, save_invstd from moments summed over the ranks (bn_moments); the running statistics take
+    the unbiased variance over the count in moments[-1], and ``nbt`` is incremented."""
+    c = (moments.shape[0] - 1) // 2
+    if moments.dtype != torch.float64 or not moments.is_cuda or not moments.is_contiguous() or moments.shape != (2 * c + 1,):
+        raise RuntimeError("bn_finalize_moments: moments must be the contiguous CUDA float64 tensor [2c + 1] of bn_moments")
+    _same_device(moments)
+    scale = torch.empty((4, c), device=moments.device, dtype=torch.float32)
+    _check(gamma, beta, running_mean, running_var)
+    if nbt is not None and nbt.dtype != torch.int64:
+        raise RuntimeError("num_batches_tracked must be int64")
+    _call("agcn_bn_finalize", None, 0, 0, c, _ptr(gamma), _ptr(beta), _ptr(running_mean), _ptr(running_var),
+          _ptr(nbt), float(momentum), float(eps), scale[0].data_ptr(), scale[1].data_ptr(), scale[2].data_ptr(), scale[3].data_ptr(),
+          2, moments.data_ptr(), _stream(), sig=(0, c, 2), work=(0.0, 0.0))
     return scale[0], scale[1], scale[2], scale[3]
 
 
@@ -387,8 +416,7 @@ def bn_stats(x, gamma, beta, running_mean, running_var, nbt, momentum, eps, trai
 
 def bn_stats_partials(x, rowmap=None):
     """Column statistics of x as mergeable partials [nparts, 4, c] (shifted sum | shifted sum of squares | pivot | row count per row
-    partition, the layout of conv_fwd_stats): the first half of a synchronised BatchNorm -- the partials of all ranks are concatenated
-    and given to bn_finalize with the global row count."""
+    partition, the layout of conv_fwd_stats): what bn_finalize, or bn_moments in a synchronised BatchNorm, reduces."""
     import ctypes
     outer, inner, ostride, c = _rowmap(x, rowmap)
     ws, nbytes = _bn_ws(c, x.device)
@@ -434,7 +462,9 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
     (eval-mode BatchNorm).  ``want_split``: dy also as bf16 pieces [2, rows, c] for conv_wgrad_presplit, None when there is no bit
     mask or c is not a multiple of 64.  ``sync`` (distributed.SyncBatchNorm, ignored when frozen): the statistics were taken over all
     ranks, so the two column sums are all-reduced between the sum pass (phase 1) and the apply pass (phase 2); dgamma / dbeta stay
-    this rank's own sums."""
+    this rank's own sums.  The rows of all ranks: ``sync.global_rows`` when the sync object has one, a CUDA float64 scalar -- the
+    count the forward's all-reduced moments carry (bn_moments), right for shards of any size; otherwise rows x sync.world (equal
+    shards)."""
     outer, inner, ostride, c = _rowmap(y, rowmap)
     if want_dy and dy is None:
         dy = torch.empty_like(y)
@@ -442,6 +472,9 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
     _check(save_mean, save_invstd, gamma)
     if pool_rows and frozen:
         raise RuntimeError("bn_bwd: the pooled tail is a training-mode path")
+    global_rows = getattr(sync, "global_rows", None) if (sync is not None and not frozen) else None
+    if global_rows is not None and (global_rows.dtype != torch.float64 or not global_rows.is_cuda or global_rows.numel() != 1):
+        raise RuntimeError("bn_bwd: sync.global_rows must be a CUDA float64 tensor with one element")
     if mask_bits is not None:
         if mask_bits.dtype != torch.int32 or not mask_bits.is_cuda:
             raise RuntimeError("bn_bwd: mask_bits must be the int32 CUDA tensor returned by bn_apply(want_mask=True)")
@@ -456,11 +489,11 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
     writes = int(dy is not None) + int(dres is not None) * (1 + int(dres_accumulate))
     pieces = int(dy_split is not None)
 
-    def run(phase, planes, sums=None, rows_all=0.0):
+    def run(phase, planes, sums=None, rows_all=None):
         # planes: the algorithmic bytes of the call in fp32 planes of y
         _call("agcn_bn_bwd", dout.data_ptr(), _ptr(mask_out), _ptr(mask_bits), y.data_ptr(), _ptr(save_mean), _ptr(save_invstd), _ptr(gamma),
               _ptr(dy), _ptr(dy_split), dgb[0].data_ptr(), dgb[1].data_ptr(), _ptr(dres), int(dres_accumulate), int(frozen),
-              outer, inner, ostride, c, int(pool_rows), phase, _ptr(sums), float(rows_all), _ptr(ws), nbytes, _stream(),
+              outer, inner, ostride, c, int(pool_rows), phase, _ptr(sums), _ptr(rows_all), _ptr(ws), nbytes, _stream(),
               sig=(outer, inner, c, mask_kind, int(pool_rows), phase, int(dy is not None), int(dres is not None), int(dres_accumulate), pieces),
               work=(0.0, 4.0 * outer * inner * c * planes))
 
@@ -469,7 +502,9 @@ def bn_bwd(dout, mask_out, y, save_mean, save_invstd, gamma, *, want_dy=True, dy
         run(1, reads)
         if dy is not None or dres is not None:
             sums = sync.all_reduce(torch.stack([dgb[1], dgb[0]]))             # (sum g | sum g xhat) over all ranks
-            run(2, reads + writes + pieces, sums, float(outer) * inner * sync.world)
+            if global_rows is None:
+                global_rows = torch.full((1,), float(outer) * inner * sync.world, device=y.device, dtype=torch.float64)
+            run(2, reads + writes + pieces, sums, global_rows)
     elif pool_rows:
         run(0, 2 + 2.0 / 32 + writes)                 # y and the bits in both passes; the pooled gradient is negligible
     else:

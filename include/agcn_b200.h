@@ -191,12 +191,20 @@ int agcn_bn_stats(const float* x, int outer, int inner, long long outer_stride, 
                   float* scale, float* shift, float* save_mean, float* save_invstd,
                   void* workspace, size_t workspace_bytes, void* stream);
 
-/* The finalize half of agcn_bn_stats (training mode) on the partials produced by agcn_conv_fwd_stats:
- * part[nparts][4][channels] (shifted sum | shifted sum of squares | pivot | row count), rows = number of rows they cover. */
+/* The finalize half of agcn_bn_stats (training mode) on the partials produced by agcn_conv_fwd_stats or agcn_bn_stats_partials:
+ * part[nparts][4][channels] (shifted sum | shifted sum of squares | pivot | row count), rows = number of rows they cover.
+ * phase 0: the whole finalize.  Phases 1 and 2 are the two halves of a synchronised BatchNorm, either side of the caller's
+ *   all-reduce of `moments` (device, fp64, [2*channels + 1], 8-byte aligned):
+ *   phase 1 reduces the partials to this rank's raw moments, moments = sum x per channel | sum x^2 per channel | rows, and writes
+ *     nothing else (no running statistics, no num_batches_tracked; gamma ... save_invstd are not read);
+ *   phase 2 reads the moments summed over the ranks, count included, and writes scale, shift, save_mean, save_invstd and the
+ *     running statistics (unbiased with the global count), and increments *num_batches_tracked; part, nparts and rows are not read.
+ *   The moments are fixed-size whatever the shard or world size, so ranks with different row counts exchange the same bytes.  */
 int agcn_bn_finalize(const float* part, int nparts, long long rows, int channels,
                      const float* gamma, const float* beta, float* running_mean, float* running_var,
                      long long* num_batches_tracked, float momentum, float eps,
-                     float* scale, float* shift, float* save_mean, float* save_invstd, void* stream);
+                     float* scale, float* shift, float* save_mean, float* save_invstd,
+                     int phase, double* moments, void* stream);
 
 /* out = act(scale*y + shift + R),  R = 0 | res | scale2*res + shift2;  act = ReLU when relu!=0.
  * (agcn.py:113-115 and :135-136).  Same addressing as agcn_bn_stats for y / res / out.
@@ -230,14 +238,15 @@ size_t agcn_bn_mask_words(int outer, int inner, int channels);
  *   broadcast over its group: dout[row][c] = dpooled[row / pool_rows][c] / pool_rows.
  * phase 0: the whole backward.  Phases 1 and 2 are the two halves of a synchronised BatchNorm, either side of the caller's
  *   all-reduce: phase 1 writes only dgamma / dbeta = this rank's sums (sum g xhat | sum g); phase 2 writes dy (dy_split, dres) from
- *   global_sums [2][channels] = (sum g | sum g xhat) all-reduced over the ranks and global_rows = the rows of all ranks.
- *   global_sums / global_rows are read in phase 2 only.
+ *   global_sums [2][channels] = (sum g | sum g xhat) all-reduced over the ranks and *global_rows = the rows of all ranks, a device
+ *   fp64 scalar (8-byte aligned; the count slot of the forward's all-reduced agcn_bn_finalize moments), so the row count never
+ *   passes through the host.  global_sums / global_rows are read in phase 2 only.
  * workspace: agcn_bn_workspace_bytes(channels).                                                                              */
 int agcn_bn_bwd(const float* dout, const float* mask_out, const unsigned* mask_bits, const float* y,
                 const float* save_mean, const float* save_invstd, const float* gamma,
                 float* dy, void* dy_split, float* dgamma, float* dbeta, float* dres, int dres_accumulate,
                 int frozen_stats, int outer, int inner, long long outer_stride, int channels, int pool_rows,
-                int phase, const float* global_sums, double global_rows,
+                int phase, const float* global_sums, const double* global_rows,
                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- pooling (agcn.py:194-196): out[g][c] = mean over rows_per_group rows of x[g][row][c] ------------ */
@@ -271,8 +280,8 @@ int agcn_bn_bwd_bits_dual(const float* dout, const unsigned* mask_bits,
  * agcn.py:44,78,83,150, computes its batch statistics over the whole batch, which a batch-sharded run only reproduces when the
  * statistics are taken over all ranks).  The collectives stay with the caller; the library provides the halves either side of them.
  * agcn_bn_stats_partials: part [nparts][4][channels] = per row partition the shifted sum | shifted sum of squares | pivot | row count
- * of x -- the layout agcn_conv_fwd_stats writes and agcn_bn_finalize merges, so the partials of all ranks are concatenated
- * (all-gather) and finalised with rows = the global row count.  The backward halves are agcn_bn_bwd phases 1 and 2.             */
+ * of x -- the layout agcn_conv_fwd_stats writes and agcn_bn_finalize merges.  Each rank reduces its own partials to fp64 moments
+ * (agcn_bn_finalize phase 1), the caller all-reduces them, and phase 2 finalises.  The backward halves are agcn_bn_bwd phases 1 and 2. */
 size_t agcn_bn_stats_partials_bytes(int channels);
 int agcn_bn_stats_partials(const float* x, int outer, int inner, long long outer_stride, int channels,
                            float* part, size_t part_bytes, int* nparts, void* workspace, size_t workspace_bytes, void* stream);
