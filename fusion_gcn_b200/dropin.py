@@ -109,14 +109,41 @@ def uninstall() -> None:
     _ORIGINALS.clear()
 
 
+def graph_step_key(model, features, label, loss_quotient=1):
+    """The key under which ``--graph-step`` caches the captured training step of ``DefaultStep.forward(model, loss_function,
+    features, label, loss_quotient)``, or None when that step has to run eagerly.
+
+    A step is graphable when the features are a CUDA tensor or a dict of CUDA tensors (the fusion models' multimodal batches),
+    the label is a CUDA tensor, ``loss_quotient >= 1``, the model is in training mode, grad mode is on and autocast is off
+    (``MixedPrecisionStep``'s ``GradScaler`` is not captured).  The key holds the model's identity, every feature entry's name,
+    shape and dtype, the label's shape and dtype and ``loss_quotient``: a replay of a graph captured under another key would
+    read the wrong model, shapes or loss scale."""
+    import torch
+    if isinstance(features, torch.Tensor):
+        entries = [(None, features)]
+    elif isinstance(features, dict) and features and all(isinstance(v, torch.Tensor) for v in features.values()):
+        entries = sorted(features.items(), key=lambda kv: str(kv[0]))
+    else:
+        return None
+    if not (all(t.is_cuda for _, t in entries) and isinstance(label, torch.Tensor) and label.is_cuda):
+        return None
+    if not (loss_quotient >= 1 and model.training and torch.is_grad_enabled()) or torch.is_autocast_enabled():
+        return None
+    return (id(model), tuple((name, tuple(t.shape), t.dtype) for name, t in entries), tuple(label.shape), label.dtype, loss_quotient)
+
+
 def _graph_steps() -> None:
     """The sessions' training step (procedures/step.py:39-46: forward, loss, backward launched op by op from Python) replayed as ONE
-    CUDA graph per step.  At the reference's own batch sizes (8 - 10, SURVEY appendix E) the eager step is launch bound: 20.8 ms against
-    11.2 ms replayed at 8 sequences (profiles/r17_bench_b8.json).  ``DefaultStep.forward`` builds a ``graphed.GraphedStep`` lazily on
-    the first training batch (BatchNorm buffers preserved across the warm-up), replays it for every batch of that shape and hands back
-    (logits, loss); ``DefaultStep.backward`` then only re-attaches the graph's static gradients (the session's ``optimizer.zero_grad()``
-    sets them to None).  Everything else -- evaluation, another batch shape (a shorter last batch), dict features of the fusion
-    models, gradient accumulation, autocast -- takes the reference's own code path."""
+    CUDA graph per step.  At the reference's own batch sizes (8 - 10, SURVEY appendix E) the eager single-tensor step is launch
+    bound: 20.8 ms against 11.2 ms replayed at 8 sequences (profiles/r17_bench_b8.json).  ``DefaultStep.forward`` builds a
+    ``graphed.GraphedStep`` lazily on the first graphable training batch (``graph_step_key``; BatchNorm buffers preserved across the
+    warm-up), replays it for every batch of that key and hands back (logits, loss / loss_quotient); ``DefaultStep.backward`` then only
+    re-attaches the graph's static gradients (the session's ``optimizer.zero_grad()`` sets them to None).  Dict features of the
+    fusion models are captured like a tensor.  With ``loss_quotient > 1`` (gradient accumulation, batch_train.py:63) the graph adds
+    each micro-batch's gradient into its static gradients: a step whose gradients are all None starts a new sum (``zero_grads()``),
+    a step whose gradients are all the graph's own adds to it, and any other state (gradients of an eager step) runs eagerly.
+    Evaluation, autocast, a second key (another model, batch shape -- a shorter last batch -- or quotient) take the reference's own
+    code path; only one graph is cached."""
     import torch
     from .graphed import GraphedStep
     importlib.import_module("session_helper")          # first, as main.py does: session <-> session_helper import each other
@@ -126,23 +153,28 @@ def _graph_steps() -> None:
 
     def forward(self, model, loss_function, features, label, loss_quotient=1):
         state["pending"] = None
-        usable = (not state["disabled"] and model.training and torch.is_grad_enabled() and isinstance(features, torch.Tensor)
-                  and features.is_cuda and label.is_cuda and loss_quotient == 1 and not torch.is_autocast_enabled())
-        if usable:
-            key = (id(model), tuple(features.shape), tuple(label.shape), features.dtype, label.dtype)
-            if state["graph"] is None:
+        key = None if state["disabled"] else graph_step_key(model, features, label, loss_quotient)
+        if key is not None:
+            trainable = [p for p in model.parameters() if p.requires_grad]
+            fresh = all(p.grad is None for p in trainable)
+            if state["graph"] is None and fresh:        # (capture resets .grad: never over gradients the session still holds)
                 try:
-                    state["graph"] = GraphedStep(model, loss_function, features, label, warmup=2, preserve_buffers=True)
+                    state["graph"] = GraphedStep(model, loss_function, features, label, warmup=2, preserve_buffers=True,
+                                                 accumulate=loss_quotient > 1, loss_divisor=loss_quotient)
                     state["key"] = key
                 except Exception as exc:                 # noqa: BLE001 -- the eager step stands in for the rest of the session
                     state["disabled"] = True
                     model.zero_grad(set_to_none=True)
                     print(f"fusion_gcn_b200.dropin: CUDA-graph step disabled ({type(exc).__name__}: {exc})", file=sys.stderr)
-            if state["graph"] is not None and key == state["key"]:
-                gs = state["graph"]
-                loss = gs(features, label)
-                state["pending"] = gs
-                return gs.logits, loss
+            gs = state["graph"]
+            if gs is not None and key == state["key"]:
+                static = {id(p): g for p, g in gs.grads}
+                if fresh and gs.accumulate:
+                    gs.zero_grads()
+                if fresh or (gs.accumulate and all(p.grad is static.get(id(p)) for p in trainable)):
+                    loss = gs(features, label)
+                    state["pending"] = gs
+                    return gs.logits, loss
         return inner_forward(self, model, loss_function, features, label, loss_quotient)
 
     def backward(self, loss):
