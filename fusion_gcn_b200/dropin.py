@@ -119,17 +119,42 @@ def graph_step_key(model, features, label, loss_quotient=1):
     shape and dtype, the label's shape and dtype and ``loss_quotient``: a replay of a graph captured under another key would
     read the wrong model, shapes or loss scale."""
     import torch
+    entries = _cuda_entries(features)
+    if entries is None or not (isinstance(label, torch.Tensor) and label.is_cuda):
+        return None
+    if not (loss_quotient >= 1 and model.training and torch.is_grad_enabled()) or torch.is_autocast_enabled():
+        return None
+    return (id(model), tuple((name, tuple(t.shape), t.dtype) for name, t in entries), tuple(label.shape), label.dtype, loss_quotient)
+
+
+def graph_eval_key(model, features):
+    """The key under which ``--graph-step`` caches the captured eval-mode forward (``graphed.GraphedForward``) of
+    ``DefaultStep.forward(model, ...)``, or None when that forward has to run eagerly.
+
+    A forward is graphable when the features are a batch-first CUDA tensor or a non-empty dict of them, the model is in eval mode,
+    grad mode is off (the sessions' ``torch.no_grad()`` validation) and autocast is off.  The key holds the model's identity and
+    every feature entry's name, trailing shape and dtype.  The batch size is not part of it: the graph serves any batch up to the
+    captured one by zero padding."""
+    import torch
+    entries = _cuda_entries(features)
+    if entries is None or any(t.dim() == 0 for _, t in entries):
+        return None
+    if model.training or torch.is_grad_enabled() or torch.is_autocast_enabled():
+        return None
+    return (id(model), tuple((name, tuple(t.shape[1:]), t.dtype) for name, t in entries))
+
+
+def _cuda_entries(features):
+    """[(name, tensor)] sorted by name (name None for a single tensor) when the features are a CUDA tensor or a non-empty dict of
+    CUDA tensors, else None."""
+    import torch
     if isinstance(features, torch.Tensor):
         entries = [(None, features)]
     elif isinstance(features, dict) and features and all(isinstance(v, torch.Tensor) for v in features.values()):
         entries = sorted(features.items(), key=lambda kv: str(kv[0]))
     else:
         return None
-    if not (all(t.is_cuda for _, t in entries) and isinstance(label, torch.Tensor) and label.is_cuda):
-        return None
-    if not (loss_quotient >= 1 and model.training and torch.is_grad_enabled()) or torch.is_autocast_enabled():
-        return None
-    return (id(model), tuple((name, tuple(t.shape), t.dtype) for name, t in entries), tuple(label.shape), label.dtype, loss_quotient)
+    return entries if all(t.is_cuda for _, t in entries) else None
 
 
 def _graph_steps() -> None:
@@ -142,14 +167,23 @@ def _graph_steps() -> None:
     fusion models are captured like a tensor.  With ``loss_quotient > 1`` (gradient accumulation, batch_train.py:63) the graph adds
     each micro-batch's gradient into its static gradients: a step whose gradients are all None starts a new sum (``zero_grads()``),
     a step whose gradients are all the graph's own adds to it, and any other state (gradients of an eager step) runs eagerly.
-    Evaluation, autocast, a second key (another model, batch shape -- a shorter last batch -- or quotient) take the reference's own
-    code path; only one graph is cached."""
+    Autocast and a second training key (another model, batch shape -- a shorter last batch -- or quotient) take the reference's own
+    code path; only one training graph is cached.
+
+    Evaluation (``validate_epoch`` and the evaluation sessions: eval mode under ``torch.no_grad()``, ``graph_eval_key``) gets a graph
+    of its own beside the training graph: a ``graphed.GraphedForward`` of the model's forward, built lazily on the first such batch
+    and replayed for every batch of that key with at most as many sequences, so a shorter last batch is zero-padded to the captured
+    size and sliced afterwards.  The step hands back a clone of the replayed logits as ``y_pred`` (the session keeps it for its
+    metrics; the next replay overwrites the graph's output) and computes ``loss_function(y_pred, label) / loss_quotient`` eagerly, as
+    the reference does.  A larger batch, another key, eval under autocast or with gradients runs eagerly; a failed eval capture is
+    reported on stderr and leaves evaluation eager for the rest of the session, the training graph untouched."""
     import torch
-    from .graphed import GraphedStep
+    from .graphed import GraphedForward, GraphedStep
     importlib.import_module("session_helper")          # first, as main.py does: session <-> session_helper import each other
     step = importlib.import_module("session.procedures.step")
     inner_forward, inner_backward = step.DefaultStep.forward, step.DefaultStep.backward
-    state = {"graph": None, "key": None, "pending": None, "disabled": False}
+    state = {"graph": None, "key": None, "pending": None, "disabled": False,
+             "eval": None, "eval_key": None, "eval_disabled": False}
 
     def forward(self, model, loss_function, features, label, loss_quotient=1):
         state["pending"] = None
@@ -175,6 +209,19 @@ def _graph_steps() -> None:
                     loss = gs(features, label)
                     state["pending"] = gs
                     return gs.logits, loss
+        eval_key = None if state["eval_disabled"] else graph_eval_key(model, features)
+        if eval_key is not None:
+            if state["eval"] is None:
+                try:
+                    state["eval"], state["eval_key"] = GraphedForward(model, features, warmup=2), eval_key
+                except Exception as exc:                 # noqa: BLE001 -- evaluation stays eager, the training graph is kept
+                    state["eval_disabled"] = True
+                    print(f"fusion_gcn_b200.dropin: CUDA-graph evaluation disabled ({type(exc).__name__}: {exc})", file=sys.stderr)
+            gf = state["eval"]
+            rows = {t.shape[0] for t in (features.values() if isinstance(features, dict) else [features])}
+            if gf is not None and eval_key == state["eval_key"] and len(rows) == 1 and 1 <= min(rows) <= gf.batch_size:
+                y_pred = gf(features).clone()
+                return y_pred, loss_function(y_pred, label) / loss_quotient
         return inner_forward(self, model, loss_function, features, label, loss_quotient)
 
     def backward(self, loss):
@@ -212,7 +259,8 @@ def main(argv=None) -> None:
     ap.add_argument("--reference", default=os.environ.get("FUSION_GCN_REFERENCE", "/root/reference"))
     ap.add_argument("--precision", default="fp32", choices=["fp32", "bf16x3", "tf32", "fp32_ffma"])
     ap.add_argument("--recompute", action="store_true", help="units recompute theta / phi and the aggregated tensor in the backward (~40 %% less activation memory)")
-    ap.add_argument("--graph-step", action="store_true", help="replay the training step (forward + loss + backward) as one CUDA graph per batch")
+    ap.add_argument("--graph-step", action="store_true", help="replay the training step (forward + loss + backward) as one CUDA graph per "
+                    "batch, and the evaluation forward (eval mode, no_grad; a shorter last batch zero-padded) as another")
     ap.add_argument("--no-dropin", action="store_true", help="run the UNMODIFIED reference under the same import shims (A/B baseline)")
     ap.add_argument("--reference-fp32", action="store_true", help="with --no-dropin: disable cuDNN / cuBLAS TF32 so the reference is an fp32 oracle (SURVEY D9)")
     ap.add_argument("--no-fused-optimizers", action="store_true", help="keep torch.optim instead of fusion_gcn_b200.optim")
